@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - headline benchmark of the SDC env-step hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): batched `sdc-v0` full-solve env, 2^20 envs per GPU, M=5, diagonal Q_delta
@@ -22,6 +22,8 @@ Timed regions
   cpu_baseline : the reference's own env (oracle/_ref/sdc_env.py, staged unmodified by `make -C oracle ref`; the numpy
           port oracle/sdc_port.py when no reference file is reachable) on one host core, ~10 s sample.
   --impl reference : the same on all host cores (multiprocessing), time-bounded samples.
+  --dump-outputs DIR : after the `value` steps, what the last of them returned (reward, flags, niter, residual, lam,
+          terminal observation planes) for a fixed sample of rank 0's envs, as float64 .npy files.
 """
 from __future__ import annotations
 
@@ -414,6 +416,28 @@ def run_secondary(torch, np, dev, rank, world, barrier, max_over_ranks, fp64_pea
     return out
 
 
+DUMP_ENVS = 1 << 17  # sampled envs per dump: 216 B each in float64 (index included), 28.3 MB in all
+
+
+def dump_outputs(path, out, N):
+    """Write what the last timed `step_tensor` returned, for a fixed seeded sample of envs, as float64 .npy files:
+    two builds run with the same arguments see the same inputs, so their dumps compare output for output."""
+    import numpy as np
+    import torch
+
+    idx = np.arange(N) if N <= DUMP_ENVS else np.sort(np.random.default_rng(0).choice(N, DUMP_ENVS, replace=False))
+    idx_dev = torch.as_tensor(idx, device=out["reward"].device)
+    arrays = {"env_index": idx.astype(np.float64)}
+    for name in ("reward", "flags", "niter", "residual"):
+        arrays[name] = out[name][idx_dev].double().cpu().numpy()
+    arrays["lam"] = torch.view_as_real(out["lam"][idx_dev]).cpu().numpy()  # (n, 2): real, imaginary part
+    if "terminal" in out:
+        arrays["terminal"] = out["terminal"][:, idx_dev].cpu().numpy()  # (4M, n) planes, as returned
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -453,10 +477,12 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for k in range(args.steps):
-        env.step_tensor(pool[k % 4])
+        out = env.step_tensor(pool[k % 4])
     e1.record()
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, N)
     launches = args.steps  # one step kernel per step (solve + reward + auto-reset fused)
     # statistics of the last step (per-rollout reduction over NCCL, outside the step path)
     niter = env.info_niter[:N].to(torch.float64)
@@ -665,7 +691,14 @@ def main():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--grid", type=int, default=4096, help="lambda grid edge of the config-4 measurement")
     ap.add_argument("--secondary-envs", type=int, default=1 << 22, help="envs per GPU of the config-3 sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0, a fixed sample of at most "
+                         f"{DUMP_ENVS} envs) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

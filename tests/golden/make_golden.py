@@ -1,4 +1,4 @@
-"""Generates tests/golden/sdc_golden.npz by running the UNMODIFIED reference env
+"""Generates tests/golden/sdc_golden_*.npz by running the UNMODIFIED reference env
 (/root/reference/sdc_gym/envs/sdc_env.py, loaded through oracle/ref_loader.py) on seeded inputs.
 
 Run in the build container only (the reference does not exist on the GPU box):
@@ -185,10 +185,24 @@ def main():
         generator="tests/golden/make_golden.py", reference="pancetta/sdc-gym sdc_gym/envs/sdc_env.py (unmodified, stub imports)",
         numpy=np.__version__, openblas=blas[0]["version"] if blas else None,
         openblas_core=blas[0]["architecture"] if blas else None, blas_variant=0, cases=cases)
-    np.savez_compressed(os.path.join(HERE, "sdc_golden.npz"), **arrays)
+    write_golden(manifest, arrays)
+    print(f"{len(cases)} cases, {sum(v.nbytes for v in arrays.values()) / 1e6:.2f} MB raw")
+
+
+SHARDS = 4  # the cases go round-robin into this many compressed files, each well under 1 MB
+
+
+def write_golden(manifest, arrays):
+    """sdc_golden_<k>.npz (arrays keyed '<case>/<array>') + sdc_golden.json (manifest; 'file' names each case's npz)"""
+    for i, case in enumerate(manifest["cases"]):
+        case["file"] = f"sdc_golden_{i % SHARDS}.npz"
+    for k in range(SHARDS):
+        fname = f"sdc_golden_{k}.npz"
+        names = {c["name"] for c in manifest["cases"] if c["file"] == fname}
+        np.savez_compressed(os.path.join(HERE, fname), **{key: v for key, v in arrays.items()
+                                                          if key.split("/", 1)[0] in names})
     with open(os.path.join(HERE, "sdc_golden.json"), "w") as f:
         json.dump(manifest, f, indent=1)
-    print(f"{len(cases)} cases, {sum(v.nbytes for v in arrays.values()) / 1e6:.2f} MB raw")
 
 
 if __name__ == "__main__":

@@ -7,24 +7,26 @@ import os
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-GOLDEN_NPZ = os.path.join(HERE, "golden", "sdc_golden.npz")
-GOLDEN_JSON = os.path.join(HERE, "golden", "sdc_golden.json")
+GOLDEN_DIR = os.path.join(HERE, "golden")
+GOLDEN_JSON = os.path.join(GOLDEN_DIR, "sdc_golden.json")
 
 _golden = None
 
 
 def golden():
+    """(manifest, {npz file name: arrays}); the manifest names the file of every case"""
     global _golden
     if _golden is None:
         with open(GOLDEN_JSON) as f:
             manifest = json.load(f)
-        arrays = np.load(GOLDEN_NPZ)
-        _golden = (manifest, arrays)
+        files = sorted({c["file"] for c in manifest["cases"]})
+        _golden = (manifest, {f: np.load(os.path.join(GOLDEN_DIR, f)) for f in files})
     return _golden
 
 
 def case_arrays(name):
-    _, arrays = golden()
+    _, files = golden()
+    arrays = files[case_meta(name)["file"]]
     prefix = name + "/"
     return {k[len(prefix):]: arrays[k] for k in arrays.files if k.startswith(prefix)}
 

@@ -1,8 +1,11 @@
-"""CPU: the `bench.py --impl reference` arm prints exactly one JSON line with the contract's keys."""
+"""`bench.py`: the `--impl reference` arm prints exactly one JSON line with the contract's keys (CPU); the arguments
+are checked (CPU); `--dump-outputs` writes the same arrays for the same arguments (GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -26,3 +29,42 @@ def test_reference_arm_json_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference"], capture_output=True,
                          text=True, env=dict(env, RANK="1", WORLD_SIZE="2"), timeout=60)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_for_the_same_arguments(tmp_path):
+    """`--dump-outputs DIR`: float64 arrays of the last timed step, identical over two runs with the same arguments"""
+    import numpy as np
+
+    dumps = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--envs-per-gpu", "5000", "--steps", "3",
+                              "--warmup", "3", "--no-secondary", "--no-cpu-baseline",
+                              "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines = [l for l in out.stdout.splitlines() if l.strip()]
+        assert len(lines) == 1
+        line = json.loads(lines[0])
+        assert line["steps"] == 3
+        dumps.append({f[:-4]: np.load(tmp_path / run / f) for f in sorted(os.listdir(tmp_path / run))})
+        # 5000 envs: the dump holds every env, so it must add up to the statistics the same run took from the env's
+        # buffers after its last timed step (a warm-up step, other envs or wrong values would not)
+        d, st = dumps[-1], line["rollout_stats"]
+        flags = d["flags"].astype(np.uint8)
+        assert d["niter"].sum() == st["sum_niter"]
+        assert np.isclose(d["reward"].sum(), st["sum_reward"], rtol=1e-12, atol=0)  # summation order differs
+        assert (flags & 2).astype(bool).sum() == st["converged"] and (flags & 4).astype(bool).sum() == st["diverged"]
+    a, b = dumps
+    assert sorted(a) == ["env_index", "flags", "lam", "niter", "residual", "reward", "terminal"]
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert a["reward"].shape == (5000,) and a["lam"].shape == (5000, 2) and a["terminal"].shape == (20, 5000)
+    assert np.array_equal(a["env_index"], np.arange(5000)) and a["niter"].min() >= 1
+    assert sorted(b) == sorted(a)
+    for k in a:
+        assert np.array_equal(a[k].view(np.int64), b[k].view(np.int64)), k
