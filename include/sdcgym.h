@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SDCGYM_ABI_VERSION 8 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_* */
+#define SDCGYM_ABI_VERSION 9 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_* */
 #define SDCGYM_MAX_M 9
 #define SDCGYM_CERT_PLANES 8
 
@@ -309,6 +309,44 @@ int sdcgym_vecnorm_reward(int64_t N, const double* reward, const uint8_t* flags,
 int sdcgym_gae(int T, int64_t N, const double* rewards, const double* values, const uint8_t* episode_starts,
                const double* last_values, const uint8_t* last_dones, double gamma, double gae_lambda,
                double* advantages, double* returns, void* stream);
+
+/*
+ * Replay buffer of an off-policy learner (SB3 ReplayBuffer + OffPolicyAlgorithm._store_transition; csrc/replay.cu).
+ * A ring of `rows` rows x N envs, every array caller-owned device memory:
+ *     obs, next_obs  [rows][P][ld]   observation planes (P = 4M, the layout of S), raw (un-normalised)
+ *     actions        [rows][N][A]    doubles; complex actions are A = 2 n_act interleaved (re, im)
+ *     rewards        [rows][N]       raw reward
+ *     dones          [rows][N]       flags & SDCGYM_FLAG_DONE
+ *     counters       [3]             pos, full (0/1), number of sample calls so far; zero-initialised by the caller
+ * The counters are read and advanced on the device only, so the calls below can be captured in a CUDA graph.
+ *   store_obs : obs[pos] = S                          (before the step: the observation the action is taken on)
+ *   store     : next_obs[pos] = DONE ? terminal : S, actions / rewards / dones[pos]; then pos += 1, wrapping to 0
+ *               and setting full.  `terminal` may be NULL when the envs are not auto-reset.  action: element (i, k)
+ *               at action[i*action_stride + k].
+ *   sample    : B transitions drawn with replacement (rows below pos, or all rows once full; envs uniformly) from the
+ *               Philox stream keyed by `seed` (csrc/replay_index.cuh), gathered as obs / next_obs planes [P][B],
+ *               actions [B][A], rewards [B], dones [B] (0.0 / 1.0), then the call counter advances.  obs_mean/obs_var
+ *               non-NULL: observations normalised as sdcgym_vecnorm_apply does; ret_var non-NULL: rewards as
+ *               sdcgym_vecnorm_reward does (same bits).  Sampling an empty buffer reads row 0.
+ */
+typedef struct sdcgym_replay {
+    int32_t P, A;
+    int64_t rows, N, ld; /* rows, N < 2^32 */
+    uint64_t seed;
+    double* obs;
+    double* next_obs;
+    double* actions;
+    double* rewards;
+    uint8_t* dones;
+    int64_t* counters;
+} sdcgym_replay;
+int sdcgym_replay_store_obs(const sdcgym_replay* rb, const double* S, int64_t s_ld, void* stream);
+int sdcgym_replay_store(const sdcgym_replay* rb, const double* S, const double* terminal, int64_t s_ld,
+                        const uint8_t* flags, const double* reward, const double* action, int64_t action_stride,
+                        void* stream);
+int sdcgym_replay_sample(const sdcgym_replay* rb, int64_t B, const double* obs_mean, const double* obs_var,
+                         const double* ret_var, double eps, double clip_obs, double clip_reward, double* obs,
+                         double* next_obs, double* actions, double* rewards, double* dones, void* stream);
 
 /*
  * Host-buffer step: `DummyVecEnv.step(actions)` with numpy-style HOST arrays on both sides, as one call.

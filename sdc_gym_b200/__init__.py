@@ -7,6 +7,8 @@ Public surface (mirrors the reference's, see DESIGN.md):
   (``SDCForceVecEnv``, ``sdc_gym/__init__.py:15-19``) composes the same kernels.
 * ``SpectralRadiusLoss`` / ``ResidualLoss`` - batched forward values of the ``dp_playground.py:186-258`` losses.
 * ``VecNormalize`` - device-side observation / reward normalisation (SB3 semantics).
+* ``RolloutBuffer`` / ``collect_rollouts`` / ``GraphedRollout`` (on-policy) and ``ReplayBuffer`` /
+  ``collect_transitions`` (off-policy) - device-resident transition storage.
 * ``collocation_matrix`` - the Gauss-Radau-right Q the reference takes from pySDC.
 
 The compute path is ``libsdcgym.so`` (hand-written CUDA, C ABI in ``include/sdcgym.h``); importing this
@@ -23,6 +25,7 @@ REGISTRY = {
 }
 
 __all__ = ["make", "make_env", "SDCVecEnv", "SDCForceVecEnv", "SpectralRadiusLoss", "ResidualLoss", "VecNormalize", "VecCheckNan", "RolloutBuffer", "collect_rollouts", "GraphedRollout",
+           "ReplayBuffer", "collect_transitions",
            "collocation_matrix", "CollGaussRadauRight", "fixed_preconditioner", "num_actions", "REGISTRY", "register_gym"]
 
 
@@ -43,6 +46,9 @@ def __getattr__(name):
     if name in ("RolloutBuffer", "collect_rollouts", "GraphedRollout"):
         from . import rollout
         return getattr(rollout, name)
+    if name in ("ReplayBuffer", "collect_transitions"):
+        from . import replay
+        return getattr(replay, name)
     raise AttributeError(name)
 
 

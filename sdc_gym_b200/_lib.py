@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SDCGYM_LIB") or os.path.join(_HERE, "libsdcgym.so")  # (SDCGYM_LIB: experiment builds)
 
 MAX_M = 9
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 ENV_KINDS = {"sdc-v0": 0, "sdc-v1": 1}
 PREC_TYPES = {"diag": 0, "lower_diag": 1, "lower_tri": 2, "strictly_lower_tri": 3, "fixed": 4}
@@ -231,6 +231,14 @@ class Xchg(ctypes.Structure):
                 ("reserved", ctypes.c_int32), ("seq", ctypes.c_uint64), ("peers", ctypes.c_void_p * MAX_RANKS)]
 
 
+class Replay(ctypes.Structure):
+    """struct sdcgym_replay"""
+
+    _fields_ = [("P", ctypes.c_int32), ("A", ctypes.c_int32), ("rows", ctypes.c_int64), ("N", ctypes.c_int64),
+                ("ld", ctypes.c_int64), ("seed", ctypes.c_uint64)] + [
+        (k, ctypes.c_void_p) for k in ("obs", "next_obs", "actions", "rewards", "dones", "counters")]
+
+
 class SdcGymError(RuntimeError):
     pass
 
@@ -313,6 +321,12 @@ def load():
         getattr(L, name).restype = ctypes.c_int
     L.sdcgym_gae.argtypes = [ctypes.c_int, i64, vp, vp, vp, vp, vp, dbl, dbl, vp, vp, vp]
     L.sdcgym_gae.restype = ctypes.c_int
+    rp = ctypes.POINTER(Replay)
+    L.sdcgym_replay_store_obs.argtypes = [rp, vp, i64, vp]
+    L.sdcgym_replay_store.argtypes = [rp, vp, vp, i64, vp, vp, vp, i64, vp]
+    L.sdcgym_replay_sample.argtypes = [rp, i64, vp, vp, vp, dbl, dbl, dbl, vp, vp, vp, vp, vp, vp]
+    for name in ("sdcgym_replay_store_obs", "sdcgym_replay_store", "sdcgym_replay_sample"):
+        getattr(L, name).restype = ctypes.c_int
     for name in ("sdcgym_residual_step", "sdcgym_vecnorm_scratch_doubles", "sdcgym_vecnorm_accumulate",
                  "sdcgym_vecnorm_merge", "sdcgym_vecnorm_update", "sdcgym_vecnorm_update_returns", "sdcgym_vecnorm_apply", "sdcgym_vecnorm_returns", "sdcgym_vecnorm_reward"):
         getattr(L, name).restype = ctypes.c_int

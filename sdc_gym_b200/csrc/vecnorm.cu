@@ -16,6 +16,7 @@
 
 #include "../../include/sdcgym.h"
 #include "bulk_copy.cuh"
+#include "normalize.cuh"
 #include "specrad.cuh"
 
 namespace sdcgym {
@@ -509,13 +510,11 @@ __global__ void __launch_bounds__(kAccThreads, 2) stat_update_kernel(const StatI
 __global__ void apply_kernel(int64_t N, int64_t ld, const double* __restrict__ X, const double* __restrict__ mean,
                              const double* __restrict__ var, double eps, double clip, double* __restrict__ Y) {
     const int p = blockIdx.y;
-    const double m = mean[p], is = 1.0 / sqrt(var[p] + eps);
+    const double m = mean[p], is = norm_inv_std(var[p], eps);
     // one 8-byte element per thread and iteration: measured 5.6 TB/s (86 % of the copy peak); a 128-bit variant
     // (two envs per access) measured 15 % slower
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
-        const double v = __dmul_rn(__dsub_rn(X[(int64_t)p * ld + i], m), is);
-        Y[(int64_t)p * ld + i] = fmin(fmax(v, -clip), clip);
-    }
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x)
+        Y[(int64_t)p * ld + i] = norm_obs(X[(int64_t)p * ld + i], m, is, clip);
 }
 
 __global__ void returns_kernel(int64_t N, const double* __restrict__ reward, double gamma, double* __restrict__ ret) {
@@ -528,7 +527,7 @@ __global__ void reward_apply_kernel(int64_t N, const double* __restrict__ reward
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
     double r = reward[i];
-    if (normalize) r = fmin(fmax(r / sqrt(ret_var[0] + eps), -clip), clip);
+    if (normalize) r = norm_reward(r, ret_var[0], eps, clip);
     out[i] = r;
     if (ret && flags && (flags[i] & SDCGYM_FLAG_DONE)) ret[i] = 0.0;
 }
