@@ -291,9 +291,43 @@ SDCGYM_HD double spectral_radius_one(const double* Q, double zr, double zi, cons
 //     d mu = y^H dK x / (y^H x),        K = z P^{-1} (Q - Qd),  P = I - z Qd
 //     dK   = z P^{-1} dQd (K - I)       =>  d mu / d Qd_ij = z conj(w_i) (mu - 1) x_j / (y^H x),   w = P^{-H} y
 //     d rho = Re( conj(mu)/|mu| d mu )  =>  g_ij = conj(mu)/|mu| * d mu / d Qd_ij   (d rho = Re(sum g_ij dQd_ij))
-// Eigenvectors come from two steps of inverse iteration on (K - mu' I) with a slightly perturbed shift; the LU
-// with partial pivoting is unrolled with predicated row swaps so everything stays in registers for small M.
+// Eigenvectors come from three steps of inverse iteration on (B - mu' I) with a slightly perturbed shift, where
+// B = D^{-1} K D is K balanced by powers of two (LAPACK zgebal without permutations).  P^{-1} grows geometrically
+// along the rows for large |z Qd|, so the entries of x and y span many orders of magnitude; on K itself their small
+// entries would carry errors of eps * max|x|, and the lower_diag / strictly_lower_tri gradients pair exactly those
+// small entries with each other.  On B they come out to a few eps each, componentwise.  The LU with partial
+// pivoting is unrolled with predicated row swaps so everything stays in registers for small M.
 // ---------------------------------------------------------------------------------------------------------
+template <int M>
+SDCGYM_HD void balance(C2 (&B)[M * M], double (&dsc)[M]) {
+#pragma unroll
+    for (int i = 0; i < M; i++) dsc[i] = 1.0;
+    bool changed = true;
+    for (int sweep = 0; sweep < 16 && changed; sweep++) {
+        changed = false;
+#pragma unroll
+        for (int i = 0; i < M; i++) {
+            double c = 0.0, r = 0.0;
+#pragma unroll
+            for (int j = 0; j < M; j++)
+                if (j != i) {
+                    c += c_abs1(B[j * M + i]);
+                    r += c_abs1(B[i * M + j]);
+                }
+            if (!(c > 0.0 && r > 0.0 && c < 1e300 && r < 1e300)) continue;
+            const int e = (ilogb(r) - ilogb(c)) / 2;  // column i times 2^e, row i times 2^-e: c 2^e ~ r 2^-e
+            const double f = ldexp(1.0, e), g = ldexp(1.0, -e);
+            if (e == 0 || !(c * f + r * g < 0.95 * (c + r))) continue;
+            changed = true;
+            dsc[i] *= f;
+#pragma unroll
+            for (int j = 0; j < M; j++) {
+                B[j * M + i] = c_scale(B[j * M + i], f);
+                B[i * M + j] = c_scale(B[i * M + j], g);
+            }
+        }
+    }
+}
 template <int M>
 SDCGYM_HD void lu_factor(C2 (&A)[M * M], int (&piv)[M]) {
 #pragma unroll
@@ -309,11 +343,13 @@ SDCGYM_HD void lu_factor(C2 (&A)[M * M], int (&piv)[M]) {
             }
         }
         piv[k] = p;
+        // swap the active columns only: the multipliers of earlier steps stay in the row order they were computed
+        // in, which is the order lu_solve applies them in (interleaved with the swaps, LINPACK dgefa/dgesl)
 #pragma unroll
         for (int q = k + 1; q < M; q++) {
             const bool sw = (p == q);
 #pragma unroll
-            for (int c = 0; c < M; c++) {
+            for (int c = k; c < M; c++) {
                 const C2 t = A[k * M + c];
                 A[k * M + c] = sw ? A[q * M + c] : t;
                 A[q * M + c] = sw ? t : A[q * M + c];
@@ -391,6 +427,8 @@ SDCGYM_HD double spectral_radius_grad_one(const double* Q, double zr, double zi,
 #pragma unroll
     for (int k = 0; k < M * M; k++) G[k] = C2{0.0, 0.0};
     if (!(rho > 1e-300) || rho != rho) return rho;  // mu = 0 (lambda = 0) or failed iteration: zero gradient
+    double dsc[M];
+    balance<M>(K, dsc);  // K <- D^{-1} K D, the same eigenvalues
     // shifted matrices: A = K - mu' I (right vector), At = A^H (left vector)
     const C2 mus = c_mul(mu, C2{1.0 + 3e-11, 2e-11});
     C2 A[M * M], At[M * M];
@@ -419,6 +457,14 @@ SDCGYM_HD double spectral_radius_grad_one(const double* Q, double zr, double zi,
         lu_solve<M>(At, pivt, y);
         normalize_vec<M>(y);
     }
+    // back to the eigenvectors of K: x = D x_B, y = D^{-1} y_B (exact: D holds powers of two)
+#pragma unroll
+    for (int i = 0; i < M; i++) {
+        x[i] = c_scale(x[i], dsc[i]);
+        y[i] = c_scale(y[i], 1.0 / dsc[i]);
+    }
+    normalize_vec<M>(x);
+    normalize_vec<M>(y);
     // w = P^{-H} y: P^H is upper triangular with entries conj(P_ji); back substitution
     C2 w[M];
 #pragma unroll

@@ -298,8 +298,12 @@ extern "C" int shim_spectral_radius_grad(const sdcgym_rho_desc* d, int64_t N, co
     switch (d->M) {
     case 2: return rho_grad_m<2>(d, N, lam, qd, rho, grad);
     case 3: return rho_grad_m<3>(d, N, lam, qd, rho, grad);
+    case 4: return rho_grad_m<4>(d, N, lam, qd, rho, grad);
     case 5: return rho_grad_m<5>(d, N, lam, qd, rho, grad);
+    case 6: return rho_grad_m<6>(d, N, lam, qd, rho, grad);
     case 7: return rho_grad_m<7>(d, N, lam, qd, rho, grad);
+    case 8: return rho_grad_m<8>(d, N, lam, qd, rho, grad);
+    case 9: return rho_grad_m<9>(d, N, lam, qd, rho, grad);
     }
     return -2;
 }
