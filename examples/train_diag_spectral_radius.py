@@ -1,9 +1,12 @@
 #!/usr/bin/env python
 """dp_playground in miniature: learn one diagonal Q_delta (the reference's `Params` "model", dp_playground.py:478-560)
-by gradient descent on the mean spectral radius over freshly sampled lambdas - forward and backward both run the
-hand-written kernels (`SpectralRadiusLoss.differentiable`).
+by gradient descent on the mean spectral radius over freshly sampled lambdas, or with --grid N over the N x N
+lambda grid of the box [-100, 0] x [-10, 0] - forward and backward both run the hand-written kernels
+(`SpectralRadiusLoss.differentiable` / `grid_differentiable`), which reduce the gradient of the one shared row on
+the device.
 
     python examples/train_diag_spectral_radius.py --M 5 --steps 300 --batch 65536
+    python examples/train_diag_spectral_radius.py --M 5 --steps 200 --grid 256
 """
 import argparse
 import os
@@ -22,6 +25,7 @@ def main(argv=None):
     ap.add_argument("--batch", type=int, default=65536)
     ap.add_argument("--lr", type=float, default=0.02)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--grid", type=int, default=0, help="train on the N x N lambda grid instead of sampled lambdas")
     args = ap.parse_args(argv)
     dev = torch.device("cuda")
     gen = torch.Generator(device=dev)
@@ -31,10 +35,13 @@ def main(argv=None):
     opt = torch.optim.Adam([theta], lr=args.lr)
     history = []
     for step in range(args.steps):
-        lam = torch.complex(torch.rand(args.batch, dtype=torch.float64, device=dev, generator=gen) * -100.0,
-                            torch.zeros(args.batch, dtype=torch.float64, device=dev))
         opt.zero_grad()
-        loss = loss_fn.differentiable(lam, theta.expand(args.batch, args.M))
+        if args.grid:
+            loss = loss_fn.grid_differentiable(args.grid, args.grid, (-100.0, 0.0), (-10.0, 0.0), theta)
+        else:
+            lam = torch.complex(torch.rand(args.batch, dtype=torch.float64, device=dev, generator=gen) * -100.0,
+                                torch.zeros(args.batch, dtype=torch.float64, device=dev))
+            loss = loss_fn.differentiable(lam, theta)
         loss.backward()
         opt.step()
         history.append(float(loss.detach()))

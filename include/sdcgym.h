@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SDCGYM_ABI_VERSION 9 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_* */
+#define SDCGYM_ABI_VERSION 10 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum */
 #define SDCGYM_MAX_M 9
 #define SDCGYM_CERT_PLANES 8
 
@@ -220,6 +220,19 @@ int sdcgym_spectral_radius(const sdcgym_rho_desc* desc, int64_t N, const double*
  */
 int sdcgym_spectral_radius_grad(const sdcgym_rho_desc* desc, int64_t N, const double* lam, const double* qd, double* rho,
                                 double* grad, void* stream);
+
+/*
+ * Sum over N samples of rho and of d rho / d theta for ONE shared parameter row (desc->qd_broadcast must be 1):
+ * sums[0] = sum rho, sums[1 + 2k], sums[2 + 2k] = sum Re g_k, sum Im g_k (g as in sdcgym_spectral_radius_grad).
+ * lam [N][2], or NULL for grid mode (grid_re/grid_im/grid_first/box as in sdcgym_spectral_radius).  rho [N] is
+ * optional (NULL: not written).  scratch: caller-owned device memory of
+ * sdcgym_spectral_radius_grad_sum_scratch_doubles(M, prec_type, N) doubles.  Deterministic: every sum is a balanced
+ * binary tree whose shape depends on N only.  A failed sample (rho NaN) makes sums[0] NaN; lambda = 0 adds zeros.
+ * N = 0 writes zeros to sums.  SDCGYM_PREC_FIXED has nothing to differentiate: SDCGYM_EUNSUPPORTED.
+ */
+int64_t sdcgym_spectral_radius_grad_sum_scratch_doubles(int M, int prec_type, int64_t N);
+int sdcgym_spectral_radius_grad_sum(const sdcgym_rho_desc* desc, int64_t N, const double* lam, const double* qd,
+                                    double* rho, double* scratch, double* sums, void* stream);
 
 /*
  * ResidualLoss.take_step (dp_playground.py:247-258) for N samples: u' = u + inv(I - lam*dt*Qd) r_old,

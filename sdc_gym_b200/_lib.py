@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SDCGYM_LIB") or os.path.join(_HERE, "libsdcgym.so")  # (SDCGYM_LIB: experiment builds)
 
 MAX_M = 9
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 ENV_KINDS = {"sdc-v0": 0, "sdc-v1": 1}
 PREC_TYPES = {"diag": 0, "lower_diag": 1, "lower_tri": 2, "strictly_lower_tri": 3, "fixed": 4}
@@ -278,6 +278,10 @@ def load():
         L.sdcgym_spectral_radius.argtypes = [ctypes.POINTER(RhoDesc), i64, vp, vp, vp, vp]
     L.sdcgym_spectral_radius_grad.argtypes = [ctypes.POINTER(RhoDesc), i64, vp, vp, vp, vp, vp]
     L.sdcgym_spectral_radius_grad.restype = ctypes.c_int
+    L.sdcgym_spectral_radius_grad_sum_scratch_doubles.argtypes = [ctypes.c_int, ctypes.c_int, i64]
+    L.sdcgym_spectral_radius_grad_sum_scratch_doubles.restype = i64
+    L.sdcgym_spectral_radius_grad_sum.argtypes = [ctypes.POINTER(RhoDesc), i64, vp, vp, vp, vp, vp, vp]
+    L.sdcgym_spectral_radius_grad_sum.restype = ctypes.c_int
     dp_ = ctypes.POINTER(RhoDesc)
     L.sdcgym_residual_step.argtypes = [dp_, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.sdcgym_vecnorm_scratch_doubles.argtypes = [ctypes.c_int]
@@ -354,4 +358,4 @@ def exported_symbols():
     header = os.path.join(os.path.dirname(_HERE), "include", "sdcgym.h")
     with open(header) as f:
         text = f.read()
-    return sorted(set(re.findall(r"\b(?:int|size_t)\s+(sdcgym_[a-z0-9_]+)\s*\(", text)))
+    return sorted(set(re.findall(r"\b(?:int|int64_t|size_t)\s+(sdcgym_[a-z0-9_]+)\s*\(", text)))

@@ -1,4 +1,4 @@
-// specrad.cu - sdcgym_spectral_radius: batched rho(K) kernel launcher (see specrad.cuh, include/sdcgym.h).
+// specrad.cu - sdcgym_spectral_radius / _grad / _grad_sum: batched rho(K) kernel launchers (see specrad.cuh, include/sdcgym.h).
 #include "specrad_params.cuh"
 
 namespace sdcgym {
@@ -15,6 +15,108 @@ template <int M>
 __global__ void __launch_bounds__(128, (M <= 5) ? 2 : 1) rho_grad_kernel(const __grid_constant__ RhoParams<M> p,
                                                                         double* __restrict__ grad) {
     rho_grad_one<M>(p, (int64_t)blockIdx.x * 128 + threadIdx.x, grad);
+}
+
+// ---- sum over samples of rho and d rho / d theta for ONE shared parameter row ------------------------------------
+// Every value is summed by a balanced binary tree whose shape depends on N alone: each 128-sample tile folds its
+// samples (5 shuffle levels per warp, then (w0 + w1) + (w2 + w3)) into one partial per value, and
+// rho_grad_sum_fold_kernel folds groups of kFold consecutive partials until one is left.  No atomics, no dependence
+// on the SM count or on timing: the same inputs give the same bits.  Padding lanes add exact zeros.
+constexpr int kFold = 256;
+
+__device__ __forceinline__ double warp_tree_sum(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    return v;  // lane 0
+}
+
+// partials [nv][T] (T = gridDim.x tiles, nv = 1 + 2 n_act values): rho, then Re / Im of each parameter's g
+template <int M>
+__global__ void __launch_bounds__(128, (M <= 5) ? 2 : 1) rho_grad_sum_kernel(const __grid_constant__ RhoParams<M> p,
+                                                                            double* __restrict__ partials) {
+    __shared__ double part[4][1 + M * (M + 1)];
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    double rho;
+    C2 G[M * M];
+    if (rho_grad_eval<M>(p, i, rho, G)) {
+        if (p.rho) p.rho[i] = rho;
+    } else {
+        rho = 0.0;
+#pragma unroll
+        for (int k = 0; k < M * M; k++) G[k] = C2{0.0, 0.0};
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    rho = warp_tree_sum(rho);
+    if (lane == 0) part[warp][0] = rho;
+    int k = 0;
+#pragma unroll
+    for (int r = 0; r < M; r++)
+#pragma unroll
+        for (int c = 0; c < M; c++) {
+            if (is_qd_param(p.prec_type, r, c)) {  // uniform over the block
+                const double gr = warp_tree_sum(G[r * M + c].r), gi = warp_tree_sum(G[r * M + c].i);
+                if (lane == 0) {
+                    part[warp][1 + 2 * k] = gr;
+                    part[warp][2 + 2 * k] = gi;
+                }
+                k++;
+            }
+        }
+    __syncthreads();
+    const int nv = 1 + 2 * p.n_act;
+    if ((int)threadIdx.x < nv) {
+        const int j = threadIdx.x;
+        partials[(int64_t)j * gridDim.x + blockIdx.x] = (part[0][j] + part[1][j]) + (part[2][j] + part[3][j]);
+    }
+}
+
+// in [nv][T] -> out [nv][ceil(T / kFold)]: block (b, j) folds in[j][b*kFold .. b*kFold + kFold) by a balanced tree
+__global__ void __launch_bounds__(kFold) rho_grad_sum_fold_kernel(int64_t T, const double* __restrict__ in,
+                                                                   double* __restrict__ out) {
+    __shared__ double part[kFold / 32];
+    const int64_t t = (int64_t)blockIdx.x * kFold + threadIdx.x;
+    const int64_t j = blockIdx.y;
+    double v = warp_tree_sum(t < T ? in[j * T + t] : 0.0);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (lane == 0) part[warp] = v;
+    __syncthreads();
+    if (warp == 0) {
+        v = lane < kFold / 32 ? part[lane] : 0.0;
+#pragma unroll
+        for (int o = kFold / 64; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+        if (lane == 0) out[j * gridDim.x + blockIdx.x] = v;
+    }
+}
+
+// Fold level sizes: T_0 = ceil(N / 128) tile partials, T_{l+1} = ceil(T_l / kFold); the fold that produces a single
+// value writes the sums, every other level lives in the scratch buffer.
+static int64_t grad_sum_scratch_values(int64_t N) {
+    int64_t T = (N + 127) / 128, total = T;
+    while (T > 1) {
+        T = (T + kFold - 1) / kFold;
+        if (T > 1) total += T;
+    }
+    return total;
+}
+
+template <int M>
+static int launch_rho_grad_sum(const sdcgym_rho_desc* d, int64_t N, const double* lam, const double* qd, double* rho,
+                               double* scratch, double* sums, cudaStream_t s) {
+    RhoParams<M> p;
+    fill_rho_params<M>(p, d, N, lam, qd, rho);
+    const int nv = 1 + 2 * p.n_act;
+    int64_t T = (N + 127) / 128;
+    rho_grad_sum_kernel<M><<<(unsigned)T, 128, 0, s>>>(p, scratch);
+    double* in = scratch;
+    while (true) {
+        const int64_t To = (T + kFold - 1) / kFold;
+        double* out = (To == 1) ? sums : in + (int64_t)nv * T;
+        rho_grad_sum_fold_kernel<<<dim3((unsigned)To, (unsigned)nv), kFold, 0, s>>>(T, in, out);
+        if (To == 1) break;
+        in = out;
+        T = To;
+    }
+    return (int)cudaGetLastError();
 }
 
 template <int M>
@@ -74,6 +176,32 @@ extern "C" int sdcgym_spectral_radius_grad(const sdcgym_rho_desc* d, int64_t N, 
     cudaStream_t s = (cudaStream_t)stream;
     switch (d->M) {
 #define C(m) case m: return launch_rho_grad<m>(d, N, lam, qd, rho, grad, s);
+        C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(9)
+#undef C
+    }
+    return SDCGYM_EUNSUPPORTED;
+}
+
+extern "C" int64_t sdcgym_spectral_radius_grad_sum_scratch_doubles(int M, int prec_type, int64_t N) {
+    if (!sdcgym_supported(M, prec_type) || prec_type == SDCGYM_PREC_FIXED) return SDCGYM_EUNSUPPORTED;
+    if (N < 0) return SDCGYM_EINVAL;
+    return (1 + 2 * (int64_t)sdcgym_num_actions(M, prec_type)) * grad_sum_scratch_values(N);
+}
+
+extern "C" int sdcgym_spectral_radius_grad_sum(const sdcgym_rho_desc* d, int64_t N, const double* lam,
+                                               const double* qd, double* rho, double* scratch, double* sums,
+                                               void* stream) {
+    if (!d || !qd || !scratch || !sums) return SDCGYM_ENULL;
+    if (!sdcgym_supported(d->M, d->prec_type) || d->prec_type == SDCGYM_PREC_FIXED) return SDCGYM_EUNSUPPORTED;
+    if (!d->qd_broadcast || N < 0) return SDCGYM_EINVAL;
+    if (N > 0 && !lam &&
+        (d->grid_re <= 0 || d->grid_im <= 0 || d->grid_first < 0 || d->grid_first + N > d->grid_re * d->grid_im))
+        return SDCGYM_EINVAL;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (N == 0)
+        return (int)cudaMemsetAsync(sums, 0, (1 + 2 * (size_t)sdcgym_num_actions(d->M, d->prec_type)) * sizeof(double), s);
+    switch (d->M) {
+#define C(m) case m: return launch_rho_grad_sum<m>(d, N, lam, qd, rho, scratch, sums, s);
         C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(9)
 #undef C
     }

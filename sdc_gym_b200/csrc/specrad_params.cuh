@@ -21,6 +21,18 @@ struct RhoParams {
     int32_t prec_type, qd_is_complex, qd_broadcast, n_act;
 };
 
+// Is the dense entry (r, c) of Q_delta a parameter of the action layout prec_type?  Parameters are numbered in
+// row-major order of the entries for which this holds.
+SDCGYM_HD bool is_qd_param(int prec_type, int r, int c) {
+    switch (prec_type) {
+    case SDCGYM_PREC_DIAG: return c == r;
+    case SDCGYM_PREC_LOWER_DIAG: return r == c + 1;
+    case SDCGYM_PREC_LOWER_TRI: return c <= r;
+    case SDCGYM_PREC_STRICTLY_LOWER_TRI: return c < r;
+    default: return false;
+    }
+}
+
 template <int M>
 SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& li, C2 (&Qd)[M * M]) {
     if (i >= p.N) return false;
@@ -42,6 +54,7 @@ SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& 
 #pragma unroll
         for (int c = 0; c < M; c++) {
             C2 d{0.0, 0.0};
+            // is_qd_param spelled out: calling it here changes the code nvcc generates for rho_kernel<8>, <9>
             bool take = false;
             switch (p.prec_type) {
             case SDCGYM_PREC_DIAG: take = (c == r); break;
@@ -70,29 +83,31 @@ SDCGYM_HD void rho_one(const RhoParams<M>& p, int64_t i) {
     p.rho[i] = spectral_radius_one<M>(p.Q, lr * p.dt, li * p.dt, Qd);
 }
 
+// rho of sample i and G = d rho / d Qd (dense, spectral_radius_grad_one); false past the end of the batch.
+template <int M>
+SDCGYM_HD bool rho_grad_eval(const RhoParams<M>& p, int64_t i, double& rho, C2 (&G)[M * M]) {
+    double lr, li;
+    C2 Qd[M * M];
+    if (!rho_inputs<M>(p, i, lr, li, Qd)) return false;
+    rho = spectral_radius_grad_one<M>(p.Q, lr * p.dt, li * p.dt, Qd, G);
+    return true;
+}
+
 // rho and d rho / d(parameter k) for the action layout of prec_type: grad[i][k] = g (complex, interleaved),
 // d rho = Re(sum_k g_k d theta_k); for real parameters the derivative is Re(g_k).
 template <int M>
 SDCGYM_HD void rho_grad_one(const RhoParams<M>& p, int64_t i, double* __restrict__ grad) {
-    double lr, li;
-    C2 Qd[M * M], G[M * M];
-    if (!rho_inputs<M>(p, i, lr, li, Qd)) return;
-    p.rho[i] = spectral_radius_grad_one<M>(p.Q, lr * p.dt, li * p.dt, Qd, G);
+    double rho;
+    C2 G[M * M];
+    if (!rho_grad_eval<M>(p, i, rho, G)) return;
+    p.rho[i] = rho;
     double* g = grad + i * (int64_t)p.n_act * 2;
     int k = 0;
 #pragma unroll
     for (int r = 0; r < M; r++)
 #pragma unroll
         for (int c = 0; c < M; c++) {
-            bool take = false;
-            switch (p.prec_type) {
-            case SDCGYM_PREC_DIAG: take = (c == r); break;
-            case SDCGYM_PREC_LOWER_DIAG: take = (r == c + 1); break;
-            case SDCGYM_PREC_LOWER_TRI: take = (c <= r); break;
-            case SDCGYM_PREC_STRICTLY_LOWER_TRI: take = (c < r); break;
-            default: break;
-            }
-            if (take) {
+            if (is_qd_param(p.prec_type, r, c)) {
                 g[2 * k] = G[r * M + c].r;
                 g[2 * k + 1] = G[r * M + c].i;
                 k++;

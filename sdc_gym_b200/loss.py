@@ -146,8 +146,114 @@ class SpectralRadiusLoss:
 
     def differentiable(self, lams, outputs):
         """Mean spectral radius as a torch scalar that supports ``.backward()`` into ``outputs`` (a CUDA tensor with
-        ``requires_grad``) - forward and backward both run the hand-written kernels."""
+        ``requires_grad``) - forward and backward both run the hand-written kernels.  A single parameter row,
+        shape (n_out,) or (1, n_out), shared by every lambda goes through ``shared_value_and_grad``."""
+        if outputs.ndim == 1 or (outputs.ndim == 2 and outputs.shape[0] == 1):
+            return _SharedRowFn.apply(outputs, lambda o, conv: self.shared_value_and_grad(lams, o, conv))
         return _SpectralRadiusFn.apply(outputs, self, lams)
+
+    def _grad_sums(self, N, lam_r, qd, is_c):
+        """(1 + 2 n_out,) CUDA float64: sum of rho, then sum Re g_k, sum Im g_k (``sdcgym_spectral_radius_grad_sum``)
+        over N samples of ONE parameter row; lam_r None selects the grid already set in the descriptor."""
+        torch = _torch()
+        d = self._desc
+        d.qd_is_complex, d.qd_broadcast = is_c, 1
+        sums = torch.empty(1 + 2 * self.n_out, dtype=torch.float64, device=self.device)
+        n_scratch = int(self._L.sdcgym_spectral_radius_grad_sum_scratch_doubles(self.M, d.prec_type, N))
+        if n_scratch < 0:
+            _lib.check(n_scratch, "sdcgym_spectral_radius_grad_sum_scratch_doubles")
+        scratch = torch.empty(n_scratch, dtype=torch.float64, device=self.device)
+        _lib.check(self._L.sdcgym_spectral_radius_grad_sum(
+            ctypes.byref(d), N, None if lam_r is None else lam_r.data_ptr(), qd.data_ptr(), None, scratch.data_ptr(),
+            sums.data_ptr(), self._stream()), "sdcgym_spectral_radius_grad_sum")
+        self._keep = (lam_r, qd, scratch)
+        return sums
+
+    def _mean_and_grad(self, sums, count, is_c, convention):
+        """(sums[0] / count, g / count) with g in ``convention`` (see ``value_and_grad``); real rows give a real g."""
+        torch = _torch()
+        if convention not in ("jax", "torch"):
+            raise ValueError("convention must be 'jax' or 'torch'")
+        pairs = sums[1:].reshape(self.n_out, 2) / max(count, 1)  # no samples: zero gradient, NaN mean
+        g = torch.view_as_complex(pairs.contiguous())
+        if not is_c:
+            g = g.real.contiguous()
+        elif convention == "torch":
+            g = g.conj().resolve_conj()
+        return sums[0] / count, g
+
+    def _shared_row(self, output):
+        if self.prec is not None:
+            raise ValueError("a fixed preconditioner has no parameters to differentiate")
+        out = output.detach() if isinstance(output, _torch().Tensor) else np.asarray(output)
+        if not (out.ndim == 1 or (out.ndim == 2 and out.shape[0] == 1)):
+            raise ValueError(f"output must be one parameter row, shape ({self.n_out},) or (1, {self.n_out})")
+        qd, is_c, _ = self._outputs_tensor(out, 1)
+        return qd, is_c
+
+    @_lib.on_device
+    def shared_value_and_grad(self, lams, output, convention="jax"):
+        """(mean rho, d mean_rho / d output) for ONE parameter row ``output`` (shape (n_out,) or (1, n_out)) shared by
+        every lambda: ``value_and_grad`` on the row expanded to the batch, reduced on the device without forming the
+        per-sample gradient (``sdcgym_spectral_radius_grad_sum``).  ``g`` has shape (n_out,); conventions as in
+        ``value_and_grad``.  An empty batch gives (NaN, zeros)."""
+        torch = _torch()
+        qd, is_c = self._shared_row(output)
+        lam = lams if isinstance(lams, torch.Tensor) else torch.as_tensor(np.asarray(lams, dtype=np.complex128))
+        lam = lam.detach().to(self.device).to(torch.complex128).reshape(-1).contiguous()
+        B = lam.numel()
+        if B == 0:  # 0/0, and nothing to launch (a NULL lambda pointer would select grid mode in the ABI)
+            sums = torch.zeros(1 + 2 * self.n_out, dtype=torch.float64, device=self.device)
+        else:
+            d = self._desc
+            d.grid_re = d.grid_im = 0
+            sums = self._grad_sums(B, torch.view_as_real(lam), qd, is_c)
+        return self._mean_and_grad(sums, B, is_c, convention)
+
+    @_lib.on_device
+    def _grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, qd, is_c, lo, hi):
+        torch = _torch()
+        N = (hi - lo) * int(n_im)
+        if N == 0:  # an empty shard contributes nothing and launches nothing
+            return torch.zeros(1 + 2 * self.n_out, dtype=torch.float64, device=self.device)
+        d = self._desc
+        d.grid_re, d.grid_im, d.grid_first = int(n_re), int(n_im), lo * int(n_im)
+        d.re_lo, d.re_hi = float(lambda_real_interval[0]), float(lambda_real_interval[1])
+        d.im_lo, d.im_hi = float(lambda_imag_interval[0]), float(lambda_imag_interval[1])
+        try:
+            return self._grad_sums(N, None, qd, is_c)
+        finally:
+            d.grid_first = 0
+
+    def grid_value_and_grad(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output, rows=None,
+                            convention="jax"):
+        """(mean rho, d mean_rho / d output) over the (n_re x n_im) lambda grid of ``grid`` for ONE parameter row,
+        lambdas generated on the device and the gradient reduced there (``sdcgym_spectral_radius_grad_sum``).
+        ``rows=None``: the whole grid, rows sharded over the ranks of the default process group as in ``grid_mean``
+        with one all-reduce of 1 + 2 n_out doubles.  ``rows=(lo, hi)``: the mean and gradient over grid rows lo..hi-1
+        only, no collective call (an empty range gives (NaN, zeros)).  Conventions as in ``value_and_grad``."""
+        qd, is_c = self._shared_row(output)
+        n_re, n_im = int(n_re), int(n_im)
+        if rows is None:
+            from . import dist as _dist
+
+            rank, world = _dist.world()
+            lo, count = _dist.shard_range(n_re, rank, world)
+            sums = self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, qd, is_c, lo, lo + count)
+            sums = _dist.all_reduce_sum(sums)
+            lo, hi = 0, n_re
+        else:
+            lo, hi = int(rows[0]), int(rows[1])
+            if not 0 <= lo <= hi <= n_re:
+                raise ValueError(f"rows={rows} outside the grid of {n_re} rows")
+            sums = self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, qd, is_c, lo, hi)
+        return self._mean_and_grad(sums, (hi - lo) * n_im, is_c, convention)
+
+    def grid_differentiable(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output):
+        """``grid_value_and_grad`` over the whole grid as a torch scalar that supports ``.backward()`` into the
+        parameter row ``output``."""
+        return _SharedRowFn.apply(output, lambda o, conv: self.grid_value_and_grad(
+            n_re, n_im, lambda_real_interval, lambda_imag_interval, o, convention=conv))
 
     @_lib.on_device
     def _sum(self, rho):
@@ -219,16 +325,39 @@ def _make_autograd_fn():
     return SpectralRadiusFn
 
 
+def _make_shared_row_fn():
+    torch = _torch()
+
+    class SharedRowFn(torch.autograd.Function):
+        """value_and_grad(row, convention) -> (scalar, g of the row's size): the loss of one shared parameter row"""
+
+        @staticmethod
+        def forward(ctx, row, value_and_grad):
+            value, g = value_and_grad(row, "torch")
+            ctx.save_for_backward(g)
+            ctx.out_shape, ctx.out_dtype = row.shape, row.dtype
+            return value.reshape(())
+
+        @staticmethod
+        def backward(ctx, upstream):
+            (g,) = ctx.saved_tensors
+            return (g * upstream).reshape(ctx.out_shape).to(ctx.out_dtype), None
+
+    return SharedRowFn
+
+
 class _LazyFn:
-    _fn = None
+    def __init__(self, make):
+        self._make, self._fn = make, None
 
     def apply(self, *a):
-        if _LazyFn._fn is None:
-            _LazyFn._fn = _make_autograd_fn()
-        return _LazyFn._fn.apply(*a)
+        if self._fn is None:
+            self._fn = self._make()
+        return self._fn.apply(*a)
 
 
-_SpectralRadiusFn = _LazyFn()
+_SpectralRadiusFn = _LazyFn(_make_autograd_fn)
+_SharedRowFn = _LazyFn(_make_shared_row_fn)
 
 NormLoss = SpectralRadiusLoss  # the reference keeps this alias (dp_playground.py:233)
 
