@@ -3,10 +3,13 @@
 by gradient descent on the mean spectral radius over freshly sampled lambdas, or with --grid N over the N x N
 lambda grid of the box [-100, 0] x [-10, 0] - forward and backward both run the hand-written kernels
 (`SpectralRadiusLoss.differentiable` / `grid_differentiable`), which reduce the gradient of the one shared row on
-the device.
+the device.  With --sweeps K it minimises instead what K sweeps of the iteration achieve,
+mean log(||r_K||_inf / ||r_0||_inf) over the sampled lambdas from the envs' reset state, with the gradient taken
+through all K sweeps (`ResidualLoss.sweeps_differentiable`).
 
     python examples/train_diag_spectral_radius.py --M 5 --steps 300 --batch 65536
     python examples/train_diag_spectral_radius.py --M 5 --steps 200 --grid 256
+    python examples/train_diag_spectral_radius.py --M 5 --steps 200 --sweeps 5
 """
 import argparse
 import os
@@ -15,7 +18,8 @@ import sys
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from sdc_gym_b200.loss import SpectralRadiusLoss  # noqa: E402
+from sdc_gym_b200.collocation import collocation_matrix  # noqa: E402
+from sdc_gym_b200.loss import ResidualLoss, SpectralRadiusLoss  # noqa: E402
 
 
 def main(argv=None):
@@ -26,17 +30,27 @@ def main(argv=None):
     ap.add_argument("--lr", type=float, default=0.02)
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--grid", type=int, default=0, help="train on the N x N lambda grid instead of sampled lambdas")
+    ap.add_argument("--sweeps", type=int, default=0,
+                    help="K > 0: minimise mean log(||r_K|| / ||r_0||) after K sweeps instead of the mean rho")
     args = ap.parse_args(argv)
     dev = torch.device("cuda")
     gen = torch.Generator(device=dev)
     gen.manual_seed(args.seed)
     loss_fn = SpectralRadiusLoss(args.M, 1.0, "diag")
+    if args.sweeps:
+        res_fn = ResidualLoss(args.M, 1.0, "diag")
+        q1 = float(abs(collocation_matrix(args.M).sum(axis=1)).max())  # ||r_0|| = |lam dt| max_i |(Q 1)_i|
     theta = torch.full((args.M,), 0.5, dtype=torch.float64, device=dev, requires_grad=True)
     opt = torch.optim.Adam([theta], lr=args.lr)
     history = []
     for step in range(args.steps):
         opt.zero_grad()
-        if args.grid:
+        if args.sweeps:
+            lam = torch.complex(torch.rand(args.batch, dtype=torch.float64, device=dev, generator=gen) * -100.0,
+                                torch.zeros(args.batch, dtype=torch.float64, device=dev))
+            n = res_fn.sweeps_differentiable(lam, theta, args.sweeps)
+            loss = torch.log(n / (lam.abs() * q1)).mean()
+        elif args.grid:
             loss = loss_fn.grid_differentiable(args.grid, args.grid, (-100.0, 0.0), (-10.0, 0.0), theta)
         else:
             lam = torch.complex(torch.rand(args.batch, dtype=torch.float64, device=dev, generator=gen) * -100.0,
@@ -46,7 +60,8 @@ def main(argv=None):
         opt.step()
         history.append(float(loss.detach()))
         if step % 50 == 0 or step == args.steps - 1:
-            print(f"step {step:4d}  mean rho {history[-1]:.6f}  diag {theta.detach().cpu().numpy().round(4)}")
+            what = f"mean log(|r_{args.sweeps}|/|r_0|)" if args.sweeps else "mean rho"
+            print(f"step {step:4d}  {what} {history[-1]:.6f}  diag {theta.detach().cpu().numpy().round(4)}")
     return history, theta.detach().cpu().numpy()
 
 

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SDCGYM_ABI_VERSION 10 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum */
+#define SDCGYM_ABI_VERSION 11 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps */
 #define SDCGYM_MAX_M 9
 #define SDCGYM_CERT_PLANES 8
 
@@ -245,6 +245,25 @@ int sdcgym_spectral_radius_grad_sum(const sdcgym_rho_desc* desc, int64_t N, cons
 int sdcgym_residual_step(const sdcgym_rho_desc* desc, int64_t N, const double* lam, const double* qd, const double* Cs,
                          const double* u0, const double* u, const double* r_old, double* u_out, double* r_out,
                          double* norm_out, double* grad, void* stream);
+
+/*
+ * ||r_K||_inf after exactly K = `sweeps` (1..50) sweeps of the iteration take_step runs, for N samples, and its gradient
+ * through all K sweeps (SDC_Fix_Env's fixed sweep count, no early stop at restol and no divergence test):
+ *     delta_k = inv(I - lam*dt*Qd) r_k,   u_{k+1} = u_k + delta_k,   r_{k+1} = u0 - (I - lam*dt*Q) u_{k+1}.
+ * lam [N] complex128 interleaved; qd as in sdcgym_spectral_radius, one row shared by every sample with
+ * desc->qd_broadcast (read in place, not expanded); u0/u/r [N][M] complex128 interleaved, or all three NULL for the
+ * envs' reset state u0 = u = 1, r = u0 - C 1 (then only lam and qd are read).  u_out/r_out [N][M] (u_K, r_K) and
+ * grad [N][A][2] are optional.  grad receives g with d norm = Re(sum_k g_k d theta_k), the derivative with respect to
+ * theta through every sweep (u0 and the incoming u, r constant); K = 1 is sdcgym_residual_step's gradient.
+ * norm_out [N]: +inf where the iteration overflowed, NaN where any component of r_K is NaN.  A norm that is 0, +inf or
+ * NaN gives g = 0.  Agreement with the reference is to rounding level, not bit-exact.
+ * Refusals, all before any CUDA call: NULL desc, lam or norm_out, or only some of u0/u/r: SDCGYM_ENULL; unsupported
+ * M / prec_type, or grad with SDCGYM_PREC_FIXED: SDCGYM_EUNSUPPORTED; N < 0 or sweeps outside 1..50: SDCGYM_EINVAL.
+ * N = 0 is a no-op.
+ */
+int sdcgym_residual_sweeps(const sdcgym_rho_desc* desc, int64_t N, int sweeps, const double* lam, const double* qd,
+                           const double* u0, const double* u, const double* r, double* u_out, double* r_out,
+                           double* norm_out, double* grad, void* stream);
 
 /*
  * Device-side VecNormalize building blocks (SB3 RunningMeanStd semantics; utils/utils.py:295-312).

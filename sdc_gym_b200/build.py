@@ -67,12 +67,14 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
     for M in M_VALUES:
         jobs.append(([nvcc, *NVCC_FLAGS, f"-DSDCGYM_M={M}", "-c", os.path.join(CSRC, "step_inst.cu"),
                       "-o", os.path.join(OBJ_DIR, f"step_m{M}.o")]))
-    for name in ("sdcgym_abi", "specrad", "vecnorm", "hostpipe", "replay"):
+    for name in ("sdcgym_abi", "specrad", "vecnorm", "hostpipe", "replay", "residual_sweeps"):
         src = os.path.join(CSRC, name + ".cu")
         if os.path.exists(src):
             # the spectral-radius kernel follows no prescribed rounding sequence: let it contract FMAs; the replay
-            # sampler is built like vecnorm.cu, whose normalisation (normalize.cuh) it shares
-            flags = [f for f in NVCC_FLAGS if not (name in ("specrad", "vecnorm", "replay") and f == "-fmad=false")]
+            # sampler is built like vecnorm.cu, whose normalisation (normalize.cuh) it shares, and so is the K-sweep
+            # residual loss, whose one-sweep counterpart lives in vecnorm.cu
+            contract = ("specrad", "vecnorm", "replay", "residual_sweeps")
+            flags = [f for f in NVCC_FLAGS if not (name in contract and f == "-fmad=false")]
             jobs.append([nvcc, *flags, "-c", src, "-o", os.path.join(OBJ_DIR, name + ".o")])
     workers = max(1, min(len(jobs), os.cpu_count() or 1))
     with concurrent.futures.ThreadPoolExecutor(workers) as ex:

@@ -346,6 +346,32 @@ def _make_shared_row_fn():
     return SharedRowFn
 
 
+def _make_sweeps_fn():
+    torch = _torch()
+
+    class SweepsFn(torch.autograd.Function):
+        """sweeps(outputs) -> (u_K, r_K, norms (B,), g (B, n_out)): per-sample norms, backward through g"""
+
+        @staticmethod
+        def forward(ctx, outputs, sweeps):
+            _, _, norms, g = sweeps(outputs)
+            g = g if outputs.is_complex() else g.real
+            ctx.save_for_backward(g.conj() if outputs.is_complex() else g)
+            ctx.out_shape, ctx.out_dtype = outputs.shape, outputs.dtype
+            return norms
+
+        @staticmethod
+        def backward(ctx, upstream):
+            (g,) = ctx.saved_tensors
+            gu = g * upstream.to(g.dtype)[:, None]
+            shared = len(ctx.out_shape) == 1 or (ctx.out_shape[0] == 1 and g.shape[0] != 1)
+            if shared:
+                gu = gu.sum(0)
+            return gu.reshape(ctx.out_shape).to(ctx.out_dtype), None
+
+    return SweepsFn
+
+
 class _LazyFn:
     def __init__(self, make):
         self._make, self._fn = make, None
@@ -358,6 +384,7 @@ class _LazyFn:
 
 _SpectralRadiusFn = _LazyFn(_make_autograd_fn)
 _SharedRowFn = _LazyFn(_make_shared_row_fn)
+_SweepsFn = _LazyFn(_make_sweeps_fn)
 
 NormLoss = SpectralRadiusLoss  # the reference keeps this alias (dp_playground.py:233)
 
@@ -407,6 +434,47 @@ class ResidualLoss:
         self._keep = (lam, qd, C, u0, u, r)
         res = (torch.view_as_complex(u_out), torch.view_as_complex(r_out), norms)
         return res + (torch.view_as_complex(grad),) if with_grad else res
+
+    @_lib.on_device
+    def sweeps(self, lams, outputs, K, u0s=None, us=None, residuals=None, with_grad=False):
+        """``(u_K, r_K, norms[, g])`` after exactly K (1..50) sweeps of ``take_step``'s iteration with C = I - z Q, no
+        early stop (``sdcgym_residual_sweeps``).  Inputs are shaped as in ``take_step``; ``u0s``, ``us`` and
+        ``residuals`` all None start from the envs' reset state u0 = u = 1, r = u0 - C 1.  ``outputs`` is (B, n_out),
+        or one row (n_out,) / (1, n_out) shared by every lambda.  ``g`` (B, n_out) complex128 is the derivative of
+        ``norms`` through all K sweeps, d norm_b = Re(sum_k g_bk d theta_bk) (for a shared row: of each sample's norm
+        with respect to that row).  A norm that is 0, +inf or NaN has g = 0."""
+        torch = _torch()
+        sr, M = self._sr, self.M
+        given = [x is not None for x in (u0s, us, residuals)]
+        if any(given) and not all(given):
+            raise ValueError("give all of u0s, us and residuals, or none of them (the reset state)")
+        lam = self._c128(lams, (-1,))
+        B = lam.shape[0]
+        out = outputs.detach() if isinstance(outputs, torch.Tensor) else outputs
+        qd, is_c, bc = sr._outputs_tensor(out, B) if B else (None, 0, 0)
+        d = sr._desc
+        d.qd_is_complex, d.qd_broadcast = is_c, bc
+        u0, u, r = (self._c128(x, (B, M)) for x in (u0s, us, residuals)) if all(given) else (None, None, None)
+        u_out = torch.empty((B, M, 2), dtype=torch.float64, device=self.device)
+        r_out = torch.empty((B, M, 2), dtype=torch.float64, device=self.device)
+        norms = torch.empty(B, dtype=torch.float64, device=self.device)
+        grad = torch.zeros((B, sr.n_out, 2), dtype=torch.float64, device=self.device) if with_grad else None
+        if B:
+            ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+            _lib.check(sr._L.sdcgym_residual_sweeps(
+                ctypes.byref(d), B, int(K), lam.data_ptr(), ptr(qd), ptr(u0), ptr(u), ptr(r), u_out.data_ptr(),
+                r_out.data_ptr(), norms.data_ptr(), ptr(grad), sr._stream()), "sdcgym_residual_sweeps")
+        self._keep = (lam, qd, u0, u, r)
+        res = (torch.view_as_complex(u_out), torch.view_as_complex(r_out), norms)
+        return res + (torch.view_as_complex(grad),) if with_grad else res
+
+    def sweeps_differentiable(self, lams, outputs, K, u0s=None, us=None, residuals=None):
+        """Per-sample ``||r_K||_inf`` (B,) of ``sweeps`` as a tensor that supports ``.backward()`` into ``outputs`` (a
+        CUDA tensor with ``requires_grad``): forward and backward both run the K-sweep kernel, and the gradient is taken
+        through every sweep.  Compose any reduction on top, e.g. ``torch.log(n).mean()``.  Real rows get a real
+        gradient, complex rows the torch convention (as ``SpectralRadiusLoss.differentiable``); a single shared row
+        gets a gradient of its own shape, summed over the batch."""
+        return _SweepsFn.apply(outputs, lambda o: self.sweeps(lams, o, K, u0s, us, residuals, with_grad=True))
 
     def __call__(self, lams, outputs, Cs, u0s, us, old_residuals):
         us_new, residuals, norms = self.take_step(lams, outputs, Cs, u0s, us, old_residuals)
