@@ -5,11 +5,13 @@ lambda grid of the box [-100, 0] x [-10, 0] - forward and backward both run the 
 (`SpectralRadiusLoss.differentiable` / `grid_differentiable`), which reduce the gradient of the one shared row on
 the device.  With --sweeps K it minimises instead what K sweeps of the iteration achieve,
 mean log(||r_K||_inf / ||r_0||_inf) over the sampled lambdas from the envs' reset state, with the gradient taken
-through all K sweeps (`ResidualLoss.sweeps_differentiable`).
+through all K sweeps (`ResidualLoss.sweeps_differentiable`); with --sweeps K --grid N it minimises that mean over the
+N x N grid, reduced on the device (`ResidualLoss.sweeps_grid_differentiable`).
 
     python examples/train_diag_spectral_radius.py --M 5 --steps 300 --batch 65536
     python examples/train_diag_spectral_radius.py --M 5 --steps 200 --grid 256
     python examples/train_diag_spectral_radius.py --M 5 --steps 200 --sweeps 5
+    python examples/train_diag_spectral_radius.py --M 5 --steps 200 --sweeps 5 --grid 256
 """
 import argparse
 import os
@@ -45,7 +47,10 @@ def main(argv=None):
     history = []
     for step in range(args.steps):
         opt.zero_grad()
-        if args.sweeps:
+        if args.sweeps and args.grid:
+            loss = res_fn.sweeps_grid_differentiable(args.grid, args.grid, (-100.0, 0.0), (-10.0, 0.0), theta,
+                                                     args.sweeps, reduction="log_ratio")
+        elif args.sweeps:
             lam = torch.complex(torch.rand(args.batch, dtype=torch.float64, device=dev, generator=gen) * -100.0,
                                 torch.zeros(args.batch, dtype=torch.float64, device=dev))
             n = res_fn.sweeps_differentiable(lam, theta, args.sweeps)

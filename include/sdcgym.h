@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SDCGYM_ABI_VERSION 11 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps */
+#define SDCGYM_ABI_VERSION 12 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps; 12: sdcgym_residual_sweeps_sum */
 #define SDCGYM_MAX_M 9
 #define SDCGYM_CERT_PLANES 8
 
@@ -264,6 +264,33 @@ int sdcgym_residual_step(const sdcgym_rho_desc* desc, int64_t N, const double* l
 int sdcgym_residual_sweeps(const sdcgym_rho_desc* desc, int64_t N, int sweeps, const double* lam, const double* qd,
                            const double* u0, const double* u, const double* r, double* u_out, double* r_out,
                            double* norm_out, double* grad, void* stream);
+
+/*
+ * Sum over N samples of a loss of ||r_K||_inf (sdcgym_residual_sweeps) and of its gradient, for ONE shared parameter
+ * row (desc->qd_broadcast must be 1, the row is read in place).  With n_K = ||r_K||_inf, n_0 = ||r_0||_inf of the
+ * starting residual (same hypot / max / NaN rule) and g the per-sample gradient of sdcgym_residual_sweeps (g = 0 where
+ * n_K is 0, +inf or NaN), each sample contributes a value f and a weighted gradient:
+ *     SDCGYM_SWEEPS_MEAN       f = n_K                g
+ *     SDCGYM_SWEEPS_LOG_RATIO  f = log(n_K / n_0)     g / n_K
+ * log_ratio: a sample with n_0 = 0 (lambda = 0 from the reset state, e.g. the corner node of a grid whose box ends at
+ * 0) contributes exact zeros to f and to the gradient; any other non-finite f (n_K = 0 gives -inf; NaN) reaches
+ * sums[0] unchanged.  sums[0] = sum f, sums[1 + 2k], sums[2 + 2k] = sum Re, sum Im of the weighted g_k: the layout of
+ * sdcgym_spectral_radius_grad_sum's sums, so the mean divides every entry by N.
+ * lam [N][2], or NULL for grid mode (grid_re/grid_im/grid_first/box as in sdcgym_spectral_radius).  u0/u/r [N][M]
+ * complex128 interleaved (list mode only), or all three NULL for the envs' reset state.  norm_out [N] (n_K) is
+ * optional.  scratch: caller-owned device memory of exactly sdcgym_spectral_radius_grad_sum_scratch_doubles(M,
+ * prec_type, N) doubles (the same tile and fold tree).  Deterministic: every sum is a balanced binary tree whose shape
+ * depends on N only.
+ * Refusals, all before any CUDA call: NULL desc, qd, scratch or sums, or only some of u0/u/r: SDCGYM_ENULL;
+ * unsupported M / prec_type, or SDCGYM_PREC_FIXED: SDCGYM_EUNSUPPORTED; qd_broadcast != 1, N < 0, sweeps outside
+ * 1..50, an unknown reduction, or in grid mode a node range outside the grid or u0/u/r given: SDCGYM_EINVAL.
+ * N = 0 writes zeros to sums.
+ */
+#define SDCGYM_SWEEPS_MEAN 0
+#define SDCGYM_SWEEPS_LOG_RATIO 1
+int sdcgym_residual_sweeps_sum(const sdcgym_rho_desc* desc, int64_t N, int sweeps, int reduction, const double* lam,
+                               const double* qd, const double* u0, const double* u, const double* r, double* norm_out,
+                               double* scratch, double* sums, void* stream);
 
 /*
  * Device-side VecNormalize building blocks (SB3 RunningMeanStd semantics; utils/utils.py:295-312).

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SDCGYM_LIB") or os.path.join(_HERE, "libsdcgym.so")  # (SDCGYM_LIB: experiment builds)
 
 MAX_M = 9
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 ENV_KINDS = {"sdc-v0": 0, "sdc-v1": 1}
 PREC_TYPES = {"diag": 0, "lower_diag": 1, "lower_tri": 2, "strictly_lower_tri": 3, "fixed": 4}
@@ -285,6 +285,7 @@ def load():
     dp_ = ctypes.POINTER(RhoDesc)
     L.sdcgym_residual_step.argtypes = [dp_, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.sdcgym_residual_sweeps.argtypes = [dp_, i64, ctypes.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.sdcgym_residual_sweeps_sum.argtypes = [dp_, i64, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.sdcgym_vecnorm_scratch_doubles.argtypes = [ctypes.c_int]
     L.sdcgym_vecnorm_accumulate.argtypes = [ctypes.c_int, i64, i64, vp, vp, vp, vp, vp]
     L.sdcgym_vecnorm_merge.argtypes = [ctypes.c_int, dbl, vp, vp, vp, vp, vp]
@@ -332,7 +333,7 @@ def load():
     L.sdcgym_replay_sample.argtypes = [rp, i64, vp, vp, vp, dbl, dbl, dbl, vp, vp, vp, vp, vp, vp]
     for name in ("sdcgym_replay_store_obs", "sdcgym_replay_store", "sdcgym_replay_sample"):
         getattr(L, name).restype = ctypes.c_int
-    for name in ("sdcgym_residual_step", "sdcgym_residual_sweeps", "sdcgym_vecnorm_scratch_doubles", "sdcgym_vecnorm_accumulate",
+    for name in ("sdcgym_residual_step", "sdcgym_residual_sweeps", "sdcgym_residual_sweeps_sum", "sdcgym_vecnorm_scratch_doubles", "sdcgym_vecnorm_accumulate",
                  "sdcgym_vecnorm_merge", "sdcgym_vecnorm_update", "sdcgym_vecnorm_update_returns", "sdcgym_vecnorm_apply", "sdcgym_vecnorm_returns", "sdcgym_vecnorm_reward"):
         getattr(L, name).restype = ctypes.c_int
     for name in ("sdcgym_num_actions", "sdcgym_supported", "sdcgym_reset", "sdcgym_step", "sdcgym_export_obs",

@@ -67,13 +67,13 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
     for M in M_VALUES:
         jobs.append(([nvcc, *NVCC_FLAGS, f"-DSDCGYM_M={M}", "-c", os.path.join(CSRC, "step_inst.cu"),
                       "-o", os.path.join(OBJ_DIR, f"step_m{M}.o")]))
-    for name in ("sdcgym_abi", "specrad", "vecnorm", "hostpipe", "replay", "residual_sweeps"):
+    for name in ("sdcgym_abi", "specrad", "vecnorm", "hostpipe", "replay", "residual_sweeps", "residual_sweeps_sum"):
         src = os.path.join(CSRC, name + ".cu")
         if os.path.exists(src):
             # the spectral-radius kernel follows no prescribed rounding sequence: let it contract FMAs; the replay
             # sampler is built like vecnorm.cu, whose normalisation (normalize.cuh) it shares, and so is the K-sweep
-            # residual loss, whose one-sweep counterpart lives in vecnorm.cu
-            contract = ("specrad", "vecnorm", "replay", "residual_sweeps")
+            # residual loss and its reduced form, whose one-sweep counterpart lives in vecnorm.cu
+            contract = ("specrad", "vecnorm", "replay", "residual_sweeps", "residual_sweeps_sum")
             flags = [f for f in NVCC_FLAGS if not (name in contract and f == "-fmad=false")]
             jobs.append([nvcc, *flags, "-c", src, "-o", os.path.join(OBJ_DIR, name + ".o")])
     workers = max(1, min(len(jobs), os.cpu_count() or 1))

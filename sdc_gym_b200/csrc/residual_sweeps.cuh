@@ -65,11 +65,36 @@ SDCGYM_HD void sweep_residual(const double (&Q)[M * M], C2 z, const C2 (&u0)[M],
     }
 }
 
-// sample i: PT the layout (SDCGYM_PREC_FIXED: p.Qd), QC complex parameters, GRAD write the gradient
-template <int M, int PT, bool QC, bool GRAD>
-SDCGYM_HD void residual_sweeps_one(const SweepParams<M>& p, int64_t i) {
-    if (i >= p.N) return;
-    const C2 z{p.lam[2 * i] * p.dt, p.lam[2 * i + 1] * p.dt};
+// The per-sample body is shared by the per-sample kernel (residual_sweeps_one) and the reduced kernel
+// (residual_sweeps_reduced): residual_sweeps_body evaluates and hands its results to an output policy `Out`, which
+// either stores them (SweepStore) or keeps what the reduction needs (SweepReduce).  The forward and reverse sweeps stay
+// in one function body, and the per-sample path forms z from lam inside it (Out::kGivenZ false): factored into
+// functions of their own, or with z passed in, nvcc generates different code for residual_sweeps_kernel.
+
+// ||r||_inf = max_a hypot(r_a): nrm, m the first index attaining it, nan_seen if any component of r is NaN (the norm
+// is then NaN)
+template <int M>
+SDCGYM_HD void sweep_norm(const C2 (&r)[M], double& nrm, int& m, bool& nan_seen) {
+    nrm = 0.0;
+    nan_seen = false;
+    m = 0;
+#pragma unroll
+    for (int a = 0; a < M; a++) {
+        const double v = hypot(r[a].r, r[a].i);
+        nan_seen |= isnan(r[a].r) || isnan(r[a].i);
+        if (v > nrm) {
+            nrm = v;
+            m = a;
+        }
+    }
+}
+
+// Out receives, in this order: start(r_0) the starting residual, norm(n_K) (NaN where r_K has a NaN), state(u_K, r_K),
+// and with GRAD grad(k, q, g_k) for each parameter k, q = its dense index r * M + c (g = 0 where n_K is 0, +inf or
+// NaN).
+template <int M, int PT, bool QC, bool GRAD, class Out>
+SDCGYM_HD void residual_sweeps_body(const SweepParams<M>& p, int64_t i, Out& out) {
+    const C2 z = Out::kGivenZ ? out.z : C2{p.lam[2 * i] * p.dt, p.lam[2 * i + 1] * p.dt};
     // zQd = z * Qd on and below the diagonal, inv[r] = 1 / P_rr
     C2 zQd[M * M], inv[M];
     constexpr int w = QC ? 2 : 1;
@@ -105,6 +130,7 @@ SDCGYM_HD void residual_sweeps_one(const SweepParams<M>& p, int64_t i) {
         for (int a = 0; a < M; a++) u0[a] = u[a] = C2{1.0, 0.0};
         sweep_residual<M>(p.Q, z, u0, u, r);
     }
+    out.start(r);
 
     C2 hist[GRAD ? kMaxSweeps * M : 1];  // delta_k, k = 0 .. K-1
     for (int s = 0; s < p.sweeps; s++) {
@@ -122,30 +148,12 @@ SDCGYM_HD void residual_sweeps_one(const SweepParams<M>& p, int64_t i) {
         sweep_residual<M>(p.Q, z, u0, u, r);
     }
 
-    double nrm = 0.0;
-    bool nan_seen = false;
-    int m = 0;
-#pragma unroll
-    for (int a = 0; a < M; a++) {
-        const double v = hypot(r[a].r, r[a].i);
-        nan_seen |= isnan(r[a].r) || isnan(r[a].i);
-        if (v > nrm) {
-            nrm = v;
-            m = a;
-        }
-    }
-    p.norm_out[i] = nan_seen ? nan("") : nrm;
-#pragma unroll
-    for (int a = 0; a < M; a++) {
-        if (p.u_out) {
-            p.u_out[(i * M + a) * 2] = u[a].r;
-            p.u_out[(i * M + a) * 2 + 1] = u[a].i;
-        }
-        if (p.r_out) {
-            p.r_out[(i * M + a) * 2] = r[a].r;
-            p.r_out[(i * M + a) * 2 + 1] = r[a].i;
-        }
-    }
+    double nrm;
+    int m;
+    bool nan_seen;
+    sweep_norm<M>(r, nrm, m, nan_seen);
+    out.norm(nan_seen ? nan("") : nrm);
+    out.state(u, r);
     if constexpr (GRAD) {
         C2 G[M * M];
 #pragma unroll
@@ -193,19 +201,98 @@ SDCGYM_HD void residual_sweeps_one(const SweepParams<M>& p, int64_t i) {
                 }
             }
         }
-        double* g = p.grad + i * (int64_t)p.n_act * 2;
         int kk = 0;
 #pragma unroll
         for (int a = 0; a < M; a++)
 #pragma unroll
             for (int c = 0; c <= a; c++)
                 if (sweep_param<PT>(a, c)) {
-                    const C2 gv = ok ? c_mul(z, G[a * M + c]) : C2{0.0, 0.0};
-                    g[2 * kk] = gv.r;
-                    g[2 * kk + 1] = gv.i;
+                    out.grad(kk, a * M + c, ok ? c_mul(z, G[a * M + c]) : C2{0.0, 0.0});
                     kk++;
                 }
     }
+}
+
+// the per-sample outputs of sdcgym_residual_sweeps: norm_out[i], optionally u_out[i], r_out[i], and grad[i] = g
+template <int M, int PT>
+struct SweepStore {
+    static constexpr bool kGivenZ = false;  // z = lam[i] dt
+    static constexpr C2 z{0.0, 0.0};
+    const SweepParams<M>& p;
+    int64_t i;
+    SDCGYM_HD void start(const C2 (&)[M]) {}
+    SDCGYM_HD void norm(double v) { p.norm_out[i] = v; }
+    SDCGYM_HD void state(const C2 (&u)[M], const C2 (&r)[M]) {
+#pragma unroll
+        for (int a = 0; a < M; a++) {
+            if (p.u_out) {
+                p.u_out[(i * M + a) * 2] = u[a].r;
+                p.u_out[(i * M + a) * 2 + 1] = u[a].i;
+            }
+            if (p.r_out) {
+                p.r_out[(i * M + a) * 2] = r[a].r;
+                p.r_out[(i * M + a) * 2 + 1] = r[a].i;
+            }
+        }
+    }
+    SDCGYM_HD void grad(int k, int, C2 gv) {
+        double* g = p.grad + i * (int64_t)p.n_act * 2;
+        g[2 * k] = gv.r;
+        g[2 * k + 1] = gv.i;
+    }
+};
+
+// sample i: PT the layout (SDCGYM_PREC_FIXED: p.Qd), QC complex parameters, GRAD write the gradient
+template <int M, int PT, bool QC, bool GRAD>
+SDCGYM_HD void residual_sweeps_one(const SweepParams<M>& p, int64_t i) {
+    if (i >= p.N) return;
+    SweepStore<M, PT> out{p, i};
+    residual_sweeps_body<M, PT, QC, GRAD>(p, i, out);
+}
+
+// Reductions of sdcgym_residual_sweeps_sum: per-sample value f and weight of g
+//   SDCGYM_SWEEPS_MEAN       f = n_K                g
+//   SDCGYM_SWEEPS_LOG_RATIO  f = log(n_K / n_0)     g / n_K
+// with n_0 = ||r_0||_inf of the starting residual (same hypot / max / NaN rule as n_K) and g = 0 where n_K is 0, +inf
+// or NaN.  log_ratio: a sample with n_0 = 0 (lambda = 0 from the reset state) contributes exact zeros to f and to the
+// gradient; any other non-finite f (n_K = 0 gives -inf, NaN) is returned as it is.
+template <int M>
+struct SweepReduce {
+    static constexpr bool kGivenZ = true;
+    C2 z;  // lambda dt, from the list or the grid
+    int reduction;
+    double n0, nK, f;
+    C2 (&gw)[M * M];  // the weighted g, dense (the caller zeroes it: entries outside the layout stay 0)
+    SDCGYM_HD void start(const C2 (&r)[M]) {
+        int m;
+        bool nan_seen;
+        sweep_norm<M>(r, n0, m, nan_seen);
+        if (nan_seen) n0 = nan("");
+    }
+    SDCGYM_HD void norm(double v) {
+        nK = v;
+        f = reduction != SDCGYM_SWEEPS_LOG_RATIO ? nK : n0 == 0.0 ? 0.0 : log(nK / n0);
+    }
+    SDCGYM_HD void state(const C2 (&)[M], const C2 (&)[M]) {}
+    SDCGYM_HD void grad(int, int q, C2 gv) {
+        if (reduction != SDCGYM_SWEEPS_LOG_RATIO)
+            gw[q] = gv;
+        else if (n0 != 0.0 && nK > 0.0 && nK <= 1.7976931348623157e308)  // elsewhere g = 0, and 0 / n_K may be NaN
+            gw[q] = c_scale(gv, 1.0 / nK);
+    }
+};
+
+// Sample i of sdcgym_residual_sweeps_sum, lambda given as z = lambda dt: returns f, sets nK = n_K (NaN where r_K has a
+// NaN) and gw = the weighted g
+template <int M, int PT, bool QC>
+SDCGYM_HD double residual_sweeps_reduced(const SweepParams<M>& p, int64_t i, C2 z, int reduction, double& nK,
+                                         C2 (&gw)[M * M]) {
+#pragma unroll
+    for (int q = 0; q < M * M; q++) gw[q] = C2{0.0, 0.0};
+    SweepReduce<M> out{z, reduction, 0.0, 0.0, 0.0, gw};
+    residual_sweeps_body<M, PT, QC, true>(p, i, out);
+    nK = out.nK;
+    return out.f;
 }
 
 template <int M>

@@ -1,5 +1,6 @@
 // specrad.cu - sdcgym_spectral_radius / _grad / _grad_sum: batched rho(K) kernel launchers (see specrad.cuh, include/sdcgym.h).
 #include "specrad_params.cuh"
+#include "tree_sum.cuh"
 
 namespace sdcgym {
 
@@ -17,19 +18,7 @@ __global__ void __launch_bounds__(128, (M <= 5) ? 2 : 1) rho_grad_kernel(const _
     rho_grad_one<M>(p, (int64_t)blockIdx.x * 128 + threadIdx.x, grad);
 }
 
-// ---- sum over samples of rho and d rho / d theta for ONE shared parameter row ------------------------------------
-// Every value is summed by a balanced binary tree whose shape depends on N alone: each 128-sample tile folds its
-// samples (5 shuffle levels per warp, then (w0 + w1) + (w2 + w3)) into one partial per value, and
-// rho_grad_sum_fold_kernel folds groups of kFold consecutive partials until one is left.  No atomics, no dependence
-// on the SM count or on timing: the same inputs give the same bits.  Padding lanes add exact zeros.
-constexpr int kFold = 256;
-
-__device__ __forceinline__ double warp_tree_sum(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-    return v;  // lane 0
-}
-
+// ---- sum over samples of rho and d rho / d theta for ONE shared parameter row (tree_sum.cuh) ----------------------
 // partials [nv][T] (T = gridDim.x tiles, nv = 1 + 2 n_act values): rho, then Re / Im of each parameter's g
 template <int M>
 __global__ void __launch_bounds__(128, (M <= 5) ? 2 : 1) rho_grad_sum_kernel(const __grid_constant__ RhoParams<M> p,
@@ -104,9 +93,12 @@ static int launch_rho_grad_sum(const sdcgym_rho_desc* d, int64_t N, const double
                                double* scratch, double* sums, cudaStream_t s) {
     RhoParams<M> p;
     fill_rho_params<M>(p, d, N, lam, qd, rho);
-    const int nv = 1 + 2 * p.n_act;
-    int64_t T = (N + 127) / 128;
+    const int64_t T = (N + 127) / 128;
     rho_grad_sum_kernel<M><<<(unsigned)T, 128, 0, s>>>(p, scratch);
+    return grad_sum_fold(T, 1 + 2 * p.n_act, scratch, sums, s);
+}
+
+int grad_sum_fold(int64_t T, int nv, double* scratch, double* sums, cudaStream_t s) {
     double* in = scratch;
     while (true) {
         const int64_t To = (T + kFold - 1) / kFold;

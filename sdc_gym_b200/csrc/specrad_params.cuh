@@ -33,6 +33,16 @@ SDCGYM_HD bool is_qd_param(int prec_type, int r, int c) {
     }
 }
 
+// lambda = lr + i li at node g of the (p.grid_re x p.grid_im) tensor grid over [p.re_lo, p.re_hi] x [p.im_lo, p.im_hi]:
+// row-major over (re, im), end points included (np.linspace semantics).  P: any parameter block with these fields
+// (read through the reference: passing them by value changes the code nvcc generates for rho_kernel).
+template <class P>
+SDCGYM_HD void grid_lambda(const P& p, int64_t g, double& lr, double& li) {
+    int64_t a = g / p.grid_im, b = g - a * p.grid_im;
+    lr = (p.grid_re > 1) ? p.re_lo + (p.re_hi - p.re_lo) * ((double)a / (double)(p.grid_re - 1)) : p.re_lo;
+    li = (p.grid_im > 1) ? p.im_lo + (p.im_hi - p.im_lo) * ((double)b / (double)(p.grid_im - 1)) : p.im_lo;
+}
+
 template <int M>
 SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& li, C2 (&Qd)[M * M]) {
     if (i >= p.N) return false;
@@ -40,11 +50,7 @@ SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& 
         lr = p.lam[2 * i];
         li = p.lam[2 * i + 1];
     } else {
-        // tensor grid, row-major over (re, im), end points included (np.linspace semantics)
-        const int64_t g = p.grid_first + i;
-        int64_t a = g / p.grid_im, b = g - a * p.grid_im;
-        lr = (p.grid_re > 1) ? p.re_lo + (p.re_hi - p.re_lo) * ((double)a / (double)(p.grid_re - 1)) : p.re_lo;
-        li = (p.grid_im > 1) ? p.im_lo + (p.im_hi - p.im_lo) * ((double)b / (double)(p.grid_im - 1)) : p.im_lo;
+        grid_lambda(p, p.grid_first + i, lr, li);
     }
     const int w = p.qd_is_complex ? 2 : 1;
     const double* row = p.qd ? p.qd + (p.qd_broadcast ? 0 : i * (int64_t)p.n_act * w) : nullptr;

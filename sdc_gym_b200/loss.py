@@ -152,17 +152,22 @@ class SpectralRadiusLoss:
             return _SharedRowFn.apply(outputs, lambda o, conv: self.shared_value_and_grad(lams, o, conv))
         return _SpectralRadiusFn.apply(outputs, self, lams)
 
+    def _sums_buffers(self, N):
+        """(sums (1 + 2 n_out,), scratch) for a device-reduced loss over N samples of ONE parameter row; the scratch
+        size is the tile and fold tree's, which ``sdcgym_residual_sweeps_sum`` shares"""
+        torch = _torch()
+        sums = torch.empty(1 + 2 * self.n_out, dtype=torch.float64, device=self.device)
+        n_scratch = int(self._L.sdcgym_spectral_radius_grad_sum_scratch_doubles(self.M, self._desc.prec_type, N))
+        if n_scratch < 0:
+            _lib.check(n_scratch, "sdcgym_spectral_radius_grad_sum_scratch_doubles")
+        return sums, torch.empty(n_scratch, dtype=torch.float64, device=self.device)
+
     def _grad_sums(self, N, lam_r, qd, is_c):
         """(1 + 2 n_out,) CUDA float64: sum of rho, then sum Re g_k, sum Im g_k (``sdcgym_spectral_radius_grad_sum``)
         over N samples of ONE parameter row; lam_r None selects the grid already set in the descriptor."""
-        torch = _torch()
         d = self._desc
         d.qd_is_complex, d.qd_broadcast = is_c, 1
-        sums = torch.empty(1 + 2 * self.n_out, dtype=torch.float64, device=self.device)
-        n_scratch = int(self._L.sdcgym_spectral_radius_grad_sum_scratch_doubles(self.M, d.prec_type, N))
-        if n_scratch < 0:
-            _lib.check(n_scratch, "sdcgym_spectral_radius_grad_sum_scratch_doubles")
-        scratch = torch.empty(n_scratch, dtype=torch.float64, device=self.device)
+        sums, scratch = self._sums_buffers(N)
         _lib.check(self._L.sdcgym_spectral_radius_grad_sum(
             ctypes.byref(d), N, None if lam_r is None else lam_r.data_ptr(), qd.data_ptr(), None, scratch.data_ptr(),
             sums.data_ptr(), self._stream()), "sdcgym_spectral_radius_grad_sum")
@@ -211,7 +216,8 @@ class SpectralRadiusLoss:
         return self._mean_and_grad(sums, B, is_c, convention)
 
     @_lib.on_device
-    def _grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, qd, is_c, lo, hi):
+    def _grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of):
+        """sums_of(N) over grid rows lo..hi-1 with the grid set in the descriptor (zeros for an empty range)"""
         torch = _torch()
         N = (hi - lo) * int(n_im)
         if N == 0:  # an empty shard contributes nothing and launches nothing
@@ -221,9 +227,25 @@ class SpectralRadiusLoss:
         d.re_lo, d.re_hi = float(lambda_real_interval[0]), float(lambda_real_interval[1])
         d.im_lo, d.im_hi = float(lambda_imag_interval[0]), float(lambda_imag_interval[1])
         try:
-            return self._grad_sums(N, None, qd, is_c)
+            return sums_of(N)
         finally:
             d.grid_first = 0
+
+    def _sharded_grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, rows, sums_of):
+        """(sums, sample count) of sums_of over the grid: ``rows=None`` shards the rows over the ranks of the default
+        process group and all-reduces the 1 + 2 n_out sums; ``rows=(lo, hi)`` takes those rows only, no collective."""
+        n_re, n_im = int(n_re), int(n_im)
+        if rows is None:
+            from . import dist as _dist
+
+            rank, world = _dist.world()
+            lo, count = _dist.shard_range(n_re, rank, world)
+            sums = self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, lo + count, sums_of)
+            return _dist.all_reduce_sum(sums), n_re * n_im
+        lo, hi = int(rows[0]), int(rows[1])
+        if not 0 <= lo <= hi <= n_re:
+            raise ValueError(f"rows={rows} outside the grid of {n_re} rows")
+        return self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of), (hi - lo) * n_im
 
     def grid_value_and_grad(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output, rows=None,
                             convention="jax"):
@@ -233,21 +255,9 @@ class SpectralRadiusLoss:
         with one all-reduce of 1 + 2 n_out doubles.  ``rows=(lo, hi)``: the mean and gradient over grid rows lo..hi-1
         only, no collective call (an empty range gives (NaN, zeros)).  Conventions as in ``value_and_grad``."""
         qd, is_c = self._shared_row(output)
-        n_re, n_im = int(n_re), int(n_im)
-        if rows is None:
-            from . import dist as _dist
-
-            rank, world = _dist.world()
-            lo, count = _dist.shard_range(n_re, rank, world)
-            sums = self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, qd, is_c, lo, lo + count)
-            sums = _dist.all_reduce_sum(sums)
-            lo, hi = 0, n_re
-        else:
-            lo, hi = int(rows[0]), int(rows[1])
-            if not 0 <= lo <= hi <= n_re:
-                raise ValueError(f"rows={rows} outside the grid of {n_re} rows")
-            sums = self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, qd, is_c, lo, hi)
-        return self._mean_and_grad(sums, (hi - lo) * n_im, is_c, convention)
+        sums, count = self._sharded_grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, rows,
+                                              lambda N: self._grad_sums(N, None, qd, is_c))
+        return self._mean_and_grad(sums, count, is_c, convention)
 
     def grid_differentiable(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output):
         """``grid_value_and_grad`` over the whole grid as a torch scalar that supports ``.backward()`` into the
@@ -388,6 +398,8 @@ _SweepsFn = _LazyFn(_make_sweeps_fn)
 
 NormLoss = SpectralRadiusLoss  # the reference keeps this alias (dp_playground.py:233)
 
+SWEEPS_REDUCTIONS = {"mean": 0, "log_ratio": 1}  # SDCGYM_SWEEPS_MEAN, SDCGYM_SWEEPS_LOG_RATIO (include/sdcgym.h)
+
 
 class ResidualLoss:
     """``dp_playground.py:235-258``: one sweep with the learned Q_delta; loss = mean ||r'||_inf.
@@ -475,6 +487,78 @@ class ResidualLoss:
         gradient, complex rows the torch convention (as ``SpectralRadiusLoss.differentiable``); a single shared row
         gets a gradient of its own shape, summed over the batch."""
         return _SweepsFn.apply(outputs, lambda o: self.sweeps(lams, o, K, u0s, us, residuals, with_grad=True))
+
+    def _sweeps_args(self, K, reduction, u0s, us, residuals):
+        if reduction not in SWEEPS_REDUCTIONS:
+            raise ValueError(f"reduction must be one of {sorted(SWEEPS_REDUCTIONS)}, not {reduction!r}")
+        given = [x is not None for x in (u0s, us, residuals)]
+        if any(given) and not all(given):
+            raise ValueError("give all of u0s, us and residuals, or none of them (the reset state)")
+        return int(K), SWEEPS_REDUCTIONS[reduction]
+
+    def _sweeps_sums(self, N, K, reduction, lam, qd, is_c, u0=None, u=None, r=None):
+        """(1 + 2 n_out,) CUDA float64 (``sdcgym_residual_sweeps_sum``) over N samples of ONE parameter row; lam None
+        selects the grid already set in the descriptor"""
+        sr = self._sr
+        d = sr._desc
+        d.qd_is_complex, d.qd_broadcast = is_c, 1
+        sums, scratch = sr._sums_buffers(N)
+        ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        _lib.check(sr._L.sdcgym_residual_sweeps_sum(
+            ctypes.byref(d), N, K, reduction, ptr(lam), qd.data_ptr(), ptr(u0), ptr(u), ptr(r), None,
+            scratch.data_ptr(), sums.data_ptr(), sr._stream()), "sdcgym_residual_sweeps_sum")
+        self._keep = (lam, qd, u0, u, r, scratch)
+        return sums
+
+    @_lib.on_device
+    def sweeps_shared_value_and_grad(self, lams, output, K, u0s=None, us=None, residuals=None, reduction="mean",
+                                     convention="jax"):
+        """(mean loss, d mean / d output) after exactly K sweeps (as ``sweeps``) for ONE parameter row ``output``
+        (shape (n_out,) or (1, n_out)) shared by every lambda, reduced on the device without forming the per-sample
+        gradient, u_K or r_K (``sdcgym_residual_sweeps_sum``).  ``reduction``: 'mean', the mean of n_K = ||r_K||_inf
+        (``ResidualLoss``'s own loss), or 'log_ratio', the mean of log(n_K / n_0) with n_0 = ||r_0||_inf of the
+        starting residual.  A sample with n_0 = 0 (lambda = 0 from the reset state) adds zeros to the log_ratio value
+        and gradient; a sample whose n_K is 0, +inf or NaN adds a zero gradient, and its value (n_K = 0: -inf under
+        log_ratio) reaches the mean unchanged.  The mean divides by the batch size.  ``g`` has shape (n_out,);
+        conventions as in ``SpectralRadiusLoss.value_and_grad``.  An empty batch gives (NaN, zeros)."""
+        torch = _torch()
+        K, red = self._sweeps_args(K, reduction, u0s, us, residuals)
+        qd, is_c = self._sr._shared_row(output)
+        lam = self._c128(lams, (-1,))
+        B = lam.shape[0]
+        if B == 0:  # 0/0, and nothing to launch (a NULL lambda pointer would select grid mode in the ABI)
+            sums = torch.zeros(1 + 2 * self._sr.n_out, dtype=torch.float64, device=self.device)
+        else:
+            self._sr._desc.grid_re = self._sr._desc.grid_im = 0
+            states = (self._c128(x, (B, self.M)) for x in (u0s, us, residuals)) if u0s is not None else ()
+            sums = self._sweeps_sums(B, K, red, lam, qd, is_c, *states)
+        return self._sr._mean_and_grad(sums, B, is_c, convention)
+
+    def sweeps_grid_value_and_grad(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output, K,
+                                   reduction="mean", rows=None, convention="jax"):
+        """``sweeps_shared_value_and_grad`` from the envs' reset state over the (n_re x n_im) lambda grid of
+        ``SpectralRadiusLoss.grid``, lambdas generated on the device.  ``rows=None``: the whole grid, rows sharded
+        over the ranks of the default process group with one all-reduce of 1 + 2 n_out doubles.  ``rows=(lo, hi)``:
+        grid rows lo..hi-1 only, no collective call (an empty range gives (NaN, zeros))."""
+        K, red = self._sweeps_args(K, reduction, None, None, None)
+        sr = self._sr
+        qd, is_c = sr._shared_row(output)
+        sums, count = sr._sharded_grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, rows,
+                                            lambda N: self._sweeps_sums(N, K, red, None, qd, is_c))
+        return sr._mean_and_grad(sums, count, is_c, convention)
+
+    def sweeps_shared_differentiable(self, lams, output, K, u0s=None, us=None, residuals=None, reduction="mean"):
+        """``sweeps_shared_value_and_grad`` as a torch scalar that supports ``.backward()`` into the parameter row
+        ``output``"""
+        return _SharedRowFn.apply(output, lambda o, conv: self.sweeps_shared_value_and_grad(
+            lams, o, K, u0s, us, residuals, reduction, conv))
+
+    def sweeps_grid_differentiable(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output, K,
+                                   reduction="mean"):
+        """``sweeps_grid_value_and_grad`` over the whole grid as a torch scalar that supports ``.backward()`` into the
+        parameter row ``output``"""
+        return _SharedRowFn.apply(output, lambda o, conv: self.sweeps_grid_value_and_grad(
+            n_re, n_im, lambda_real_interval, lambda_imag_interval, o, K, reduction, convention=conv))
 
     def __call__(self, lams, outputs, Cs, u0s, us, old_residuals):
         us_new, residuals, norms = self.take_step(lams, outputs, Cs, u0s, us, old_residuals)
