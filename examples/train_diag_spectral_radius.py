@@ -6,12 +6,15 @@ lambda grid of the box [-100, 0] x [-10, 0] - forward and backward both run the 
 the device.  With --sweeps K it minimises instead what K sweeps of the iteration achieve,
 mean log(||r_K||_inf / ||r_0||_inf) over the sampled lambdas from the envs' reset state, with the gradient taken
 through all K sweeps (`ResidualLoss.sweeps_differentiable`); with --sweeps K --grid N it minimises that mean over the
-N x N grid, reduced on the device (`ResidualLoss.sweeps_grid_differentiable`).
+N x N grid, reduced on the device (`ResidualLoss.sweeps_grid_differentiable`).  With --eval-grid N it then judges the
+trained row as the reference does, by sdc-v0 iteration counts and success rate, over the N x N grid next to MIN's
+(`IterationCounts.grid_summary`).
 
     python examples/train_diag_spectral_radius.py --M 5 --steps 300 --batch 65536
     python examples/train_diag_spectral_radius.py --M 5 --steps 200 --grid 256
     python examples/train_diag_spectral_radius.py --M 5 --steps 200 --sweeps 5
     python examples/train_diag_spectral_radius.py --M 5 --steps 200 --sweeps 5 --grid 256
+    python examples/train_diag_spectral_radius.py --M 5 --steps 200 --grid 256 --eval-grid 512
 """
 import argparse
 import os
@@ -34,6 +37,8 @@ def main(argv=None):
     ap.add_argument("--grid", type=int, default=0, help="train on the N x N lambda grid instead of sampled lambdas")
     ap.add_argument("--sweeps", type=int, default=0,
                     help="K > 0: minimise mean log(||r_K|| / ||r_0||) after K sweeps instead of the mean rho")
+    ap.add_argument("--eval-grid", type=int, default=0,
+                    help="N > 0: after training, print the sdc-v0 iteration counts of the row and of MIN on the N x N grid")
     args = ap.parse_args(argv)
     dev = torch.device("cuda")
     gen = torch.Generator(device=dev)
@@ -67,6 +72,17 @@ def main(argv=None):
         if step % 50 == 0 or step == args.steps - 1:
             what = f"mean log(|r_{args.sweeps}|/|r_0|)" if args.sweeps else "mean rho"
             print(f"step {step:4d}  {what} {history[-1]:.6f}  diag {theta.detach().cpu().numpy().round(4)}")
+    if args.eval_grid:
+        # the reference's judgement of the trained row: sdc-v0 iteration counts and success rate, here over every
+        # lambda of the N x N grid, next to MIN's
+        from sdc_gym_b200.iterations import IterationCounts
+
+        n, box = args.eval_grid, ((-100.0, 0.0), (-10.0, 0.0))
+        for name, ev, row in (("MIN", IterationCounts(args.M, 1.0, 1e-10, prec="min"), None),
+                              ("RL", IterationCounts(args.M, 1.0, 1e-10, "diag"), theta.detach())):
+            s = ev.grid_summary(n, n, *box, row)
+            print(f"{name:<3} -- Mean number of iterations and success rate: {s.mean_niter:4.2f}, "
+                  f"{s.success_rate * 100} %")
     return history, theta.detach().cpu().numpy()
 
 

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SDCGYM_ABI_VERSION 12 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps; 12: sdcgym_residual_sweeps_sum */
+#define SDCGYM_ABI_VERSION 13 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps; 12: sdcgym_residual_sweeps_sum; 13: sdcgym_full_solve_counts */
 #define SDCGYM_MAX_M 9
 #define SDCGYM_CERT_PLANES 8
 
@@ -179,6 +179,36 @@ int sdcgym_reset(const sdcgym_env_desc* desc, const sdcgym_state* st, const doub
 /* env.step(action) for all N envs (sdc_env.py:209-273 / 507-572), plus the DummyVecEnv auto-reset when
  * desc->autoreset != 0. */
 int sdcgym_step(const sdcgym_env_desc* desc, const sdcgym_state* st, const sdcgym_step_io* io, void* stream);
+
+/*
+ * The sdc-v0 full solve (sdc_env.py:209-273) of N nodes from the reset state, without any env state: what
+ * sdcgym_reset(lam_in) followed by sdcgym_step gives for each node, bit for bit, but nothing is read or written besides
+ * lambda, the action rows and the outputs below.  The evaluation of a Q_delta by its iteration counts
+ * (rl_playground.py:147-156, dp_playground.py:844-957).
+ *   desc     env_kind SDCGYM_ENV_FULL; M, prec_type, Q, Qd_fixed, dt, restol, max_iters, action_is_complex, do_scale and
+ *            blas_variant as for sdcgym_step (the reward, seed and sampling fields are not used)
+ *   grid     NULL: node i has lambda lam[2i] + i lam[2i+1].  Else node i is grid node first + i of the (n_re x n_im)
+ *            tensor grid over [re_lo, re_hi] x [im_lo, im_hi], row-major over (re, im), end points included: the same
+ *            bits as the nodes of sdcgym_spectral_radius / sdcgym_residual_sweeps_sum in grid mode.
+ *   action   element (node i, component k) at action[i*a_es + k*a_cs] (+1 = imag), a_es = 0 for one row shared by
+ *            every node; NULL with SDCGYM_PREC_FIXED
+ *   outputs  each optional (NULL: not written): niter_out [N] int32 (info['niter']), residual_out [N] (info['residual']),
+ *            flags_out [N] SDCGYM_FLAG_*, lam_out [N][2] (the lambda each node ran with)
+ *   hist     optional, int64 [max_iters + 3], zeroed by the call: [0, max_iters] the niter of the converged nodes,
+ *            [max_iters + 1] the number of err nodes, [max_iters + 2] the nodes that ran out of sweeps unconverged
+ * Refusals, all before any CUDA call: NULL desc: SDCGYM_ENULL; env_kind != SDCGYM_ENV_FULL, or an unsupported M,
+ * prec_type or blas_variant: SDCGYM_EUNSUPPORTED; N > 0 without actions for a learned prec_type, or without lam in list
+ * mode: SDCGYM_ENULL; actions with SDCGYM_PREC_FIXED, per-node rows (a_es != 0) in grid mode, N < 0, max_iters outside
+ * 0..16384, or a grid range outside the grid: SDCGYM_EINVAL.  N = 0 only zeroes hist.  No host synchronisation: the
+ * call can be captured in a CUDA graph.
+ */
+typedef struct sdcgym_lambda_grid {
+    int64_t n_re, n_im, first;
+    double re_lo, re_hi, im_lo, im_hi;
+} sdcgym_lambda_grid;
+int sdcgym_full_solve_counts(const sdcgym_env_desc* desc, const sdcgym_lambda_grid* grid, int64_t N, const double* lam,
+                             const double* action, int64_t a_es, int64_t a_cs, int32_t* niter_out, double* residual_out,
+                             uint8_t* flags_out, double* lam_out, int64_t* hist, void* stream);
 
 /* planes S[4M][ld] -> reference observation layout obs[N][2][M] complex128 (interleaved re, im) and back */
 int sdcgym_export_obs(int M, int64_t N, int64_t ld, const double* S, double* obs, void* stream);

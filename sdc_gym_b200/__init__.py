@@ -6,6 +6,8 @@ Public surface (mirrors the reference's, see DESIGN.md):
   DummyVecEnv protocol (reference ``sdc_gym/__init__.py:3-13``, ``utils/utils.py:235-315``); ``sdc-v4``
   (``SDCForceVecEnv``, ``sdc_gym/__init__.py:15-19``) composes the same kernels.
 * ``SpectralRadiusLoss`` / ``ResidualLoss`` - batched forward values of the ``dp_playground.py:186-258`` losses.
+* ``IterationCounts`` - iteration counts and success rate of the ``sdc-v0`` full solve over a lambda batch or grid
+  (the reference's ``test_model`` evaluation), counted on the device.
 * ``VecNormalize`` - device-side observation / reward normalisation (SB3 semantics).
 * ``RolloutBuffer`` / ``collect_rollouts`` / ``GraphedRollout`` (on-policy) and ``ReplayBuffer`` /
   ``collect_transitions`` (off-policy) - device-resident transition storage.
@@ -24,7 +26,7 @@ REGISTRY = {
     "sdc-v4": ("SDC_Full_Force_Env", 50),  # sdc_gym/__init__.py:15-19 (force_env.py)
 }
 
-__all__ = ["make", "make_env", "SDCVecEnv", "SDCForceVecEnv", "SpectralRadiusLoss", "ResidualLoss", "VecNormalize", "VecCheckNan", "RolloutBuffer", "collect_rollouts", "GraphedRollout",
+__all__ = ["make", "make_env", "SDCVecEnv", "SDCForceVecEnv", "SpectralRadiusLoss", "ResidualLoss", "IterationCounts", "VecNormalize", "VecCheckNan", "RolloutBuffer", "collect_rollouts", "GraphedRollout",
            "ReplayBuffer", "collect_transitions",
            "collocation_matrix", "CollGaussRadauRight", "fixed_preconditioner", "num_actions", "REGISTRY", "register_gym"]
 
@@ -40,6 +42,9 @@ def __getattr__(name):
     if name in ("SpectralRadiusLoss", "ResidualLoss"):
         from . import loss
         return getattr(loss, name)
+    if name in ("IterationCounts", "CountSummary"):
+        from . import iterations
+        return getattr(iterations, name)
     if name in ("VecNormalize", "VecCheckNan"):
         from . import vec_normalize
         return getattr(vec_normalize, name)

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SDCGYM_LIB") or os.path.join(_HERE, "libsdcgym.so")  # (SDCGYM_LIB: experiment builds)
 
 MAX_M = 9
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 ENV_KINDS = {"sdc-v0": 0, "sdc-v1": 1}
 PREC_TYPES = {"diag": 0, "lower_diag": 1, "lower_tri": 2, "strictly_lower_tri": 3, "fixed": 4}
@@ -126,6 +126,14 @@ class RhoDesc(ctypes.Structure):
         ("im_lo", ctypes.c_double),
         ("im_hi", ctypes.c_double),
     ]
+
+
+class LambdaGrid(ctypes.Structure):
+    """struct sdcgym_lambda_grid"""
+
+    _fields_ = [("n_re", ctypes.c_int64), ("n_im", ctypes.c_int64), ("first", ctypes.c_int64),
+                ("re_lo", ctypes.c_double), ("re_hi", ctypes.c_double), ("im_lo", ctypes.c_double),
+                ("im_hi", ctypes.c_double)]
 
 
 class HostIO(ctypes.Structure):
@@ -286,6 +294,9 @@ def load():
     L.sdcgym_residual_step.argtypes = [dp_, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.sdcgym_residual_sweeps.argtypes = [dp_, i64, ctypes.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.sdcgym_residual_sweeps_sum.argtypes = [dp_, i64, ctypes.c_int, ctypes.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.sdcgym_full_solve_counts.argtypes = [ctypes.POINTER(EnvDesc), ctypes.POINTER(LambdaGrid), i64, vp, vp, i64, i64,
+                                           vp, vp, vp, vp, vp, vp]
+    L.sdcgym_full_solve_counts.restype = ctypes.c_int
     L.sdcgym_vecnorm_scratch_doubles.argtypes = [ctypes.c_int]
     L.sdcgym_vecnorm_accumulate.argtypes = [ctypes.c_int, i64, i64, vp, vp, vp, vp, vp]
     L.sdcgym_vecnorm_merge.argtypes = [ctypes.c_int, dbl, vp, vp, vp, vp, vp]

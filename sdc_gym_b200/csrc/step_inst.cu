@@ -277,9 +277,79 @@ static cudaError_t launch_certified_diag(const StepParams<kM>& p, const FastWork
     return cudaGetLastError();
 }
 
+// sdcgym_full_solve_counts: the per-thread kernel of launch_step at HoldPolicy's residency for every M (the team kernel
+// and the phased solve give the same bits and are not used), plus the histogram behind the side store
+template <int V, bool DENSE>
+static cudaError_t launch_full_solve_counts(const StepParams<kM>& p, const ResetEval& src, int64_t* hist, cudaStream_t s) {
+    constexpr int hold = DENSE ? kHoldDense : kHoldDiag;
+    constexpr int minb = DENSE ? HoldPolicy<kM>::dense_minb : HoldPolicy<kM>::diag_minb;
+    constexpr int block = DENSE ? HoldPolicy<kM>::dense_block : HoldPolicy<kM>::diag_block;
+    const size_t smem = step_kernel_smem_bytes<kM, hold, block>() + (hist ? (size_t)(p.max_iters + 3) * sizeof(int) : 0);
+    auto kernel = full_solve_counts_kernel<kM, V, DENSE, hold, minb, block>;
+    if (smem > 48 * 1024) {
+        // per-device opt-in, raised when a call needs more than the largest size granted so far
+        static std::atomic<size_t> granted[64];
+        int dev = 0;
+        cudaError_t e = cudaGetDevice(&dev);
+        if (e != cudaSuccess) return e;
+        if (dev < 0 || dev >= 64 || granted[dev].load(std::memory_order_relaxed) < smem) {
+            e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+            if (dev >= 0 && dev < 64) granted[dev].store(smem, std::memory_order_relaxed);
+        }
+    }
+    kernel<<<(unsigned)((p.N + block - 1) / block), block, smem, s>>>(p, src, reinterpret_cast<unsigned long long*>(hist));
+    return cudaGetLastError();
+}
+
 }  // namespace sdcgym
 
 using namespace sdcgym;
+
+extern "C" int SDCGYM_CAT(sdcgym_launch_full_solve_counts_m, SDCGYM_M)(
+    const sdcgym_env_desc* d, const sdcgym_lambda_grid* g, int64_t N, const double* lam, const double* action,
+    int64_t a_es, int64_t a_cs, int32_t* niter_out, double* residual_out, uint8_t* flags_out, double* lam_out,
+    int64_t* hist, void* stream) {
+    sdcgym_state st{};  // no env state: every plane NULL
+    st.N = st.ld = N;
+    StepParams<kM> p;
+    fill_params<kM>(p, d, &st);
+    p.action = action;
+    p.a_es = a_es;
+    p.a_cs = a_cs;
+    p.info_niter = niter_out;
+    p.info_res = residual_out;
+    p.flags = flags_out;
+    p.info_lam = lam_out;
+    p.autoreset = 0;
+    p.strategy = SDCGYM_REW_ITERATION_ONLY;
+    ResetEval src{};
+    src.lam = g ? nullptr : lam;
+    if (g) {
+        src.grid_re = g->n_re;
+        src.grid_im = g->n_im;
+        src.grid_first = g->first;
+        src.re_lo = g->re_lo;
+        src.re_hi = g->re_hi;
+        src.im_lo = g->im_lo;
+        src.im_hi = g->im_hi;
+    }
+    bool dense = d->prec_type != SDCGYM_PREC_DIAG;
+    if (d->prec_type == SDCGYM_PREC_FIXED) {  // a fixed diagonal matrix takes the diagonal kernel, as in sdcgym_step
+        bool diagonal = true;
+        for (int r = 0; r < kM; r++)
+            for (int c = 0; c < kM; c++)
+                if (r != c && d->Qd_fixed[r * kM + c] != 0.0) diagonal = false;
+        dense = !diagonal;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    cudaError_t e;
+    if (d->blas_variant == SDCGYM_BLAS_SKYLAKEX)
+        e = dense ? launch_full_solve_counts<0, true>(p, src, hist, s) : launch_full_solve_counts<0, false>(p, src, hist, s);
+    else
+        e = dense ? launch_full_solve_counts<1, true>(p, src, hist, s) : launch_full_solve_counts<1, false>(p, src, hist, s);
+    return (int)e;
+}
 
 extern "C" int SDCGYM_CAT(sdcgym_launch_reset_m, SDCGYM_M)(const sdcgym_env_desc* d, const sdcgym_state* st,
                                                           const double* lam_in, const uint8_t* mask, double* old_states,

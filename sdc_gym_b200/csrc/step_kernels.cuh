@@ -368,6 +368,48 @@ struct NoAfterLoads {
     SDCGYM_HD void operator()() const {}
 };
 
+// Where a full solve starts from and what it leaves behind.  EnvPlanes (default): the env's own state planes
+// (StepParams::lam, S, resnorm, ...), read at the start and written back at the end, with the reward and the auto-reset.
+struct EnvPlanes {
+    static constexpr bool kEval = false;
+    SDCGYM_HD void lambda(int64_t, double&, double&) const {}
+    SDCGYM_HD void count(bool, int, bool, bool, int) const {}
+};
+
+// Evaluation of the sdc-v0 full solve from the reset state (sdcgym_full_solve_counts): lambda from an interleaved list
+// or the node of a tensor grid, (u, r) and ||r0|| from the statements of reset_one, and no state planes at all - no
+// reward, no terminal state, no auto-reset.  The results leave through StepParams::info_niter / info_res / flags /
+// info_lam; `hist` (shared memory of the block, or nullptr) counts the outcome of every valid thread:
+// [0, max_iters] niter of the converged nodes, max_iters + 1 err, max_iters + 2 out of sweeps.
+struct ResetEval {
+    static constexpr bool kEval = true;
+    const double* lam;  // [N][2], or nullptr: node grid_first + i of the grid below
+    int64_t grid_re, grid_im, grid_first;
+    double re_lo, re_hi, im_lo, im_hi;
+    int* hist;
+    // grid_lambda (specrad_params.cuh) as the translation units built with contraction compile it: one FMA, spelled out
+    // here because this unit is built with -fmad=false
+    SDCGYM_HD void lambda(int64_t i, double& lr, double& li) const {
+        if (lam) {
+            lr = lam[2 * i];
+            li = lam[2 * i + 1];
+            return;
+        }
+        const int64_t g = grid_first + i, a = g / grid_im, b = g - a * grid_im;
+        lr = (grid_re > 1) ? dfma(dsub(re_hi, re_lo), ddiv((double)a, (double)(grid_re - 1)), re_lo) : re_lo;
+        li = (grid_im > 1) ? dfma(dsub(im_hi, im_lo), ddiv((double)b, (double)(grid_im - 1)), im_lo) : im_lo;
+    }
+    SDCGYM_HD void count(bool valid, int it, bool conv, bool err, int max_iters) const {
+        if (!hist || !valid) return;
+        const int bin = err ? max_iters + 1 : (conv ? it : max_iters + 2);
+#ifdef __CUDA_ARCH__
+        atomicAdd(hist + bin, 1);
+#else
+        hist[bin]++;
+#endif
+    }
+};
+
 // `after_loads` runs once every input of the env sits in registers (non-dense kernels): the streaming kernel releases
 // its shared-memory stage there and starts the next tile's copies.
 //
@@ -380,10 +422,14 @@ struct NoAfterLoads {
 // resnorm plane keeps the norm the divergence test compares against), the inverse to p.pinv_scratch (first pass only)
 // and its index to p.cont_list; a PHASE 2 pass picks it up with exactly those bits, so the sweep sequence of every
 // env - and therefore every output - is the one of the single-launch kernel.  PHASE 0 = no phases (unchanged code).
-template <int M, int KIND, int V, bool DENSE, int HOLD, class AfterLoads = NoAfterLoads, int PHASE = 0>
+// Src: EnvPlanes, or ResetEval (sdc-v0 full solve from the reset state, PHASE 0, no StepInputs).
+template <int M, int KIND, int V, bool DENSE, int HOLD, class AfterLoads = NoAfterLoads, int PHASE = 0,
+          class Src = EnvPlanes>
 SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side = nullptr, const int side_stride = 1,
                         cplx* pside = nullptr, const int pstride = 1, const StepInputs* in = nullptr,
-                        AfterLoads after_loads = AfterLoads(), const uint32_t taddr = 0) {
+                        AfterLoads after_loads = AfterLoads(), const uint32_t taddr = 0, const Src& src = Src()) {
+    constexpr bool kEval = Src::kEval;
+    static_assert(!kEval || (KIND == SDCGYM_ENV_FULL && PHASE == 0 && HOLD != 10), "evaluation: single-launch full solve");
     const bool valid = tid < p.N;
     const int64_t i = valid ? tid : p.N - 1;
     const int64_t ld = p.ld;
@@ -395,7 +441,13 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
     // ---- phase 0: every global load of this env is issued here, in one basic block, so that a single DRAM round trip
     //      covers them all (placed at their uses they end up behind the branches of the division slow paths, one
     //      exposed latency each) ----
-    double lr = in_lam[ii], li = in_lam[ild + ii];
+    double lr, li;
+    if constexpr (kEval) {
+        src.lambda(i, lr, li);
+    } else {
+        lr = in_lam[ii];
+        li = in_lam[ild + ii];
+    }
     double araw[DENSE ? 1 : M], aimg[DENSE ? 1 : M];
     if (!DENSE) {
 #pragma unroll
@@ -439,8 +491,9 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
             ri[m] = in_S[(2 * M + 2 * m + 1) * ild + ii];
         }
     };
-    if (!DENSE) load_state();  // the dense kernels need the registers for the inverse first
-    double nr_old = in ? in->resnorm[ii] : p.resnorm[i];
+    if (!DENSE && !kEval) load_state();  // the dense kernels need the registers for the inverse first
+    // (evaluation: the reset state is derived from lambda once z is known, below)
+    double nr_old = kEval ? 0.0 : (in ? in->resnorm[ii] : p.resnorm[i]);
     static_assert(PHASE == 0 || (DENSE && KIND == SDCGYM_ENV_FULL && HOLD != 5), "phased launches: dense full solves");
     int it = (KIND == SDCGYM_ENV_STEP || PHASE == 2) ? (in ? in->niter[ii] : p.niter[i]) : 0;
     // the auto-reset needs these at the very end
@@ -462,8 +515,10 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
         //  which the compiler does not move shared-memory loads across; listing it cost the sdc-v0 kernel 2 %)
 #pragma unroll
         for (int k = 0; k < M; k++) asm volatile("" : "+d"(araw[k]), "+d"(aimg[k]));
+        if constexpr (!kEval) {
 #pragma unroll
-        for (int m = 0; m < M; m++) asm volatile("" : "+d"(ur[m]), "+d"(ui[m]), "+d"(rr[m]), "+d"(ri[m]));
+            for (int m = 0; m < M; m++) asm volatile("" : "+d"(ur[m]), "+d"(ui[m]), "+d"(rr[m]), "+d"(ri[m]));
+        }
     }
 #endif
     if (!DENSE) after_loads();
@@ -671,7 +726,13 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
 #endif
 
 
-    if (DENSE) load_state();
+    if constexpr (kEval) {
+        // reset_one's statements: u = 1, r = u0 - C u, ||r0||
+        initial_state<M, V>(p.Q, zr, zi, ur, ui, rr, ri);
+        nr_old = inf_norm_fast<M>(rr, ri);
+    } else if (DENSE) {
+        load_state();
+    }
 
     // sdc-v1 needs the previous residual for the reward when norm_factor != 1
     double norm_old_scaled = nr_old;
@@ -871,8 +932,10 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
     }
 
     // ---- reward ----
-    double rew;
-    if (err) {
+    double rew = 0.0;
+    if constexpr (kEval) {
+        src.count(valid, it, conv, err, p.max_iters);
+    } else if (err) {
         rew = dmul(-p.step_penalty, (double)(p.max_iters + 1));
     } else if (p.strategy == SDCGYM_REW_ITERATION_ONLY) {
         rew = dmul((double)(-it), p.step_penalty);
@@ -905,6 +968,7 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
         p.info_lam[2 * i] = lr;  // interleaved complex128, directly viewable by the host layer
         p.info_lam[2 * i + 1] = li;
     }
+    if constexpr (kEval) return;
     if (KIND == SDCGYM_ENV_STEP && p.old_states && it < p.max_iters)
         store_column<M>(p.old_states, i, p.max_iters, it, ur, ui, rr, ri);
 
@@ -1016,11 +1080,45 @@ __global__ void __launch_bounds__(kBlock, MINB) inverse_kernel(const __grid_cons
 }
 
 template <int M, int HOLD, int BLOCK = kBlock>
-constexpr size_t step_kernel_smem_bytes() {
+__host__ __device__ constexpr size_t step_kernel_smem_bytes() {
     return HOLD == 3 ? (size_t)M * M * BLOCK * sizeof(double)
                      : ((HOLD == 4 || HOLD == 7 || HOLD == 8 || HOLD == 9) ? (size_t)2 * M * M * BLOCK * sizeof(double)
                                   : (HOLD == 5 ? (size_t)4 * M * M * BLOCK * sizeof(double)
                                                : (HOLD == 6 ? (size_t)M * M * BLOCK * sizeof(double) : 0)));
+}
+
+// sdcgym_full_solve_counts: step_kernel's full solve from the reset state (step_one with ResetEval).  With `hist`
+// (int64 [max_iters + 3]) the block counts its outcomes in shared memory behind the side store and adds each non-zero
+// bin to `hist` once: integer sums, so the result does not depend on the order of the blocks.
+template <int M, int V, bool DENSE, int HOLD, int MINB, int BLOCK>
+__global__ void __launch_bounds__(BLOCK, MINB) full_solve_counts_kernel(const __grid_constant__ StepParams<M> p,
+                                                                        const __grid_constant__ ResetEval src,
+                                                                        unsigned long long* __restrict__ hist) {
+    extern __shared__ double2 eval_smem[];  // [side store of HOLD][BLOCK], then the block's histogram (int)
+    constexpr size_t kSide = step_kernel_smem_bytes<M, HOLD, BLOCK>() / sizeof(double2);
+    const int nbins = p.max_iters + 3;
+    ResetEval ev = src;
+    ev.hist = hist ? reinterpret_cast<int*>(eval_smem + kSide) : nullptr;
+    if (hist) {
+        for (int k = threadIdx.x; k < nbins; k += BLOCK) ev.hist[k] = 0;
+        __syncthreads();
+    }
+    const int64_t tid = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
+    if constexpr (HOLD == 5 || HOLD == 7) {
+        step_one<M, SDCGYM_ENV_FULL, V, DENSE, HOLD, NoAfterLoads, 0, ResetEval>(
+            p, tid, nullptr, 1, reinterpret_cast<cplx*>(eval_smem) + threadIdx.x, BLOCK, nullptr, NoAfterLoads(), 0, ev);
+    } else if constexpr (HOLD >= 3) {
+        step_one<M, SDCGYM_ENV_FULL, V, DENSE, HOLD, NoAfterLoads, 0, ResetEval>(
+            p, tid, reinterpret_cast<double*>(eval_smem) + threadIdx.x, BLOCK, nullptr, 1, nullptr, NoAfterLoads(), 0, ev);
+    } else {
+        step_one<M, SDCGYM_ENV_FULL, V, DENSE, HOLD, NoAfterLoads, 0, ResetEval>(p, tid, nullptr, 1, nullptr, 1, nullptr,
+                                                                                 NoAfterLoads(), 0, ev);
+    }
+    if (hist) {
+        __syncthreads();  // (every thread comes back from step_one: its exits are returns of the inlined body)
+        for (int k = threadIdx.x; k < nbins; k += BLOCK)
+            if (ev.hist[k]) atomicAdd(hist + k, (unsigned long long)ev.hist[k]);
+    }
 }
 #endif
 

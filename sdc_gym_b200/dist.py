@@ -57,6 +57,21 @@ def all_reduce_sum(t):
     return t
 
 
+def sharded_rows_sum(n_rows, rows, sums_of):
+    """(sums, number of rows summed) of ``sums_of(lo, hi)``, a tensor of sums over the rows lo..hi-1 of a grid of
+    ``n_rows`` rows.  ``rows=None``: this rank's ``shard_range`` of the rows, the sums all-reduced over the default
+    process group (every rank gets the sums over all rows); ``rows=(lo, hi)``: those rows only, no collective call."""
+    n_rows = int(n_rows)
+    if rows is None:
+        rank, size = world()
+        lo, count = shard_range(n_rows, rank, size)
+        return all_reduce_sum(sums_of(lo, lo + count)), n_rows
+    lo, hi = int(rows[0]), int(rows[1])
+    if not 0 <= lo <= hi <= n_rows:
+        raise ValueError(f"rows={rows} outside the grid of {n_rows} rows")
+    return sums_of(lo, hi), hi - lo
+
+
 class PeerExchange:
     """Exchange regions for the in-kernel all-reduce of the normaliser moments (include/sdcgym.h ``sdcgym_xchg``):
     every rank allocates one region, the 64-byte CUDA IPC handles travel over the process group (the only use of the

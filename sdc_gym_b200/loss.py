@@ -234,18 +234,12 @@ class SpectralRadiusLoss:
     def _sharded_grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, rows, sums_of):
         """(sums, sample count) of sums_of over the grid: ``rows=None`` shards the rows over the ranks of the default
         process group and all-reduces the 1 + 2 n_out sums; ``rows=(lo, hi)`` takes those rows only, no collective."""
-        n_re, n_im = int(n_re), int(n_im)
-        if rows is None:
-            from . import dist as _dist
+        from . import dist as _dist
 
-            rank, world = _dist.world()
-            lo, count = _dist.shard_range(n_re, rank, world)
-            sums = self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, lo + count, sums_of)
-            return _dist.all_reduce_sum(sums), n_re * n_im
-        lo, hi = int(rows[0]), int(rows[1])
-        if not 0 <= lo <= hi <= n_re:
-            raise ValueError(f"rows={rows} outside the grid of {n_re} rows")
-        return self._grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of), (hi - lo) * n_im
+        n_re, n_im = int(n_re), int(n_im)
+        sums, n_rows = _dist.sharded_rows_sum(n_re, rows, lambda lo, hi: self._grid_sums(
+            n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of))
+        return sums, n_rows * n_im
 
     def grid_value_and_grad(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output, rows=None,
                             convention="jax"):
