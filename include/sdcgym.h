@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SDCGYM_ABI_VERSION 13 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps; 12: sdcgym_residual_sweeps_sum; 13: sdcgym_full_solve_counts */
+#define SDCGYM_ABI_VERSION 14 /* 5: sweep_mode + work buffers in sdcgym_state; 6: in-kernel peer-memory statistics exchange; 7: sdcgym_state.norm_init; 8: sdcgym_state.phase_*; 9: sdcgym_replay_*; 10: sdcgym_spectral_radius_grad_sum; 11: sdcgym_residual_sweeps; 12: sdcgym_residual_sweeps_sum; 13: sdcgym_full_solve_counts; 14: sdcgym_full_solve_counts_population, sdcgym_spectral_radius_grad_sum_population */
 #define SDCGYM_MAX_M 9
 #define SDCGYM_CERT_PLANES 8
 
@@ -210,6 +210,20 @@ int sdcgym_full_solve_counts(const sdcgym_env_desc* desc, const sdcgym_lambda_gr
                              const double* action, int64_t a_es, int64_t a_cs, int32_t* niter_out, double* residual_out,
                              uint8_t* flags_out, double* lam_out, int64_t* hist, void* stream);
 
+/*
+ * sdcgym_full_solve_counts' histogram for each of P action rows, every row shared by all N nodes: hist int64
+ * [P][max_iters + 3], row p at action + p*a_rs (component k at + k*a_cs, +1 = imag).  hist[p] equals, bit for bit,
+ * the histogram of sdcgym_full_solve_counts(desc, grid, N, lam, action + p*a_rs, a_es = 0, a_cs) (one launch, row p =
+ * blockIdx.y; P above 65535 takes several launches).  No per-node outputs.
+ * Refusals, all before any CUDA call: NULL desc, hist or action, or N > 0 without lam in list mode: SDCGYM_ENULL;
+ * env_kind != SDCGYM_ENV_FULL, SDCGYM_PREC_FIXED, or an unsupported M, prec_type or blas_variant: SDCGYM_EUNSUPPORTED;
+ * P < 1, N < 0, max_iters outside 0..16384, or a grid range outside the grid: SDCGYM_EINVAL.  N = 0 only zeroes hist.
+ * No host synchronisation: the call can be captured in a CUDA graph.
+ */
+int sdcgym_full_solve_counts_population(const sdcgym_env_desc* desc, const sdcgym_lambda_grid* grid, int64_t N,
+                                        const double* lam, int64_t P, const double* action, int64_t a_rs,
+                                        int64_t a_cs, int64_t* hist, void* stream);
+
 /* planes S[4M][ld] -> reference observation layout obs[N][2][M] complex128 (interleaved re, im) and back */
 int sdcgym_export_obs(int M, int64_t N, int64_t ld, const double* S, double* obs, void* stream);
 int sdcgym_import_obs(int M, int64_t N, int64_t ld, const double* obs, double* S, void* stream);
@@ -263,6 +277,20 @@ int sdcgym_spectral_radius_grad(const sdcgym_rho_desc* desc, int64_t N, const do
 int64_t sdcgym_spectral_radius_grad_sum_scratch_doubles(int M, int prec_type, int64_t N);
 int sdcgym_spectral_radius_grad_sum(const sdcgym_rho_desc* desc, int64_t N, const double* lam, const double* qd,
                                     double* rho, double* scratch, double* sums, void* stream);
+
+/*
+ * sdcgym_spectral_radius_grad_sum for each of P parameter rows, every row shared by all N samples: row p at
+ * qd + p*qd_rs doubles (desc->qd_broadcast must be 1, qd_is_complex as for the single row), sums [P][1 + 2A].
+ * sums[p] equals, bit for bit, the sums of sdcgym_spectral_radius_grad_sum on row p: per row, the same tile tree
+ * and fold tree.  scratch: caller-owned device memory of P * sdcgym_spectral_radius_grad_sum_scratch_doubles(M,
+ * prec_type, N) doubles.  P above 65535 / (1 + 2A) rows takes several launches.
+ * Refusals, all before any CUDA call: NULL desc, qd, scratch or sums: SDCGYM_ENULL; unsupported M / prec_type, or
+ * SDCGYM_PREC_FIXED: SDCGYM_EUNSUPPORTED; qd_broadcast != 1, P < 1, N < 0, or in grid mode a node range outside the
+ * grid: SDCGYM_EINVAL.  N = 0 writes zeros to sums.  No host synchronisation.
+ */
+int sdcgym_spectral_radius_grad_sum_population(const sdcgym_rho_desc* desc, int64_t N, const double* lam, int64_t P,
+                                               const double* qd, int64_t qd_rs, double* scratch, double* sums,
+                                               void* stream);
 
 /*
  * ResidualLoss.take_step (dp_playground.py:247-258) for N samples: u' = u + inv(I - lam*dt*Qd) r_old,

@@ -26,7 +26,7 @@ REGISTRY = {
     "sdc-v4": ("SDC_Full_Force_Env", 50),  # sdc_gym/__init__.py:15-19 (force_env.py)
 }
 
-__all__ = ["make", "make_env", "SDCVecEnv", "SDCForceVecEnv", "SpectralRadiusLoss", "ResidualLoss", "IterationCounts", "VecNormalize", "VecCheckNan", "RolloutBuffer", "collect_rollouts", "GraphedRollout",
+__all__ = ["make", "make_env", "SDCVecEnv", "SDCForceVecEnv", "SpectralRadiusLoss", "ResidualLoss", "IterationCounts", "PopulationSummary", "VecNormalize", "VecCheckNan", "RolloutBuffer", "collect_rollouts", "GraphedRollout",
            "ReplayBuffer", "collect_transitions",
            "collocation_matrix", "CollGaussRadauRight", "fixed_preconditioner", "num_actions", "REGISTRY", "register_gym"]
 
@@ -42,7 +42,7 @@ def __getattr__(name):
     if name in ("SpectralRadiusLoss", "ResidualLoss"):
         from . import loss
         return getattr(loss, name)
-    if name in ("IterationCounts", "CountSummary"):
+    if name in ("IterationCounts", "CountSummary", "PopulationSummary"):
         from . import iterations
         return getattr(iterations, name)
     if name in ("VecNormalize", "VecCheckNan"):

@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SDCGYM_LIB") or os.path.join(_HERE, "libsdcgym.so")  # (SDCGYM_LIB: experiment builds)
 
 MAX_M = 9
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 ENV_KINDS = {"sdc-v0": 0, "sdc-v1": 1}
 PREC_TYPES = {"diag": 0, "lower_diag": 1, "lower_tri": 2, "strictly_lower_tri": 3, "fixed": 4}
@@ -297,6 +297,11 @@ def load():
     L.sdcgym_full_solve_counts.argtypes = [ctypes.POINTER(EnvDesc), ctypes.POINTER(LambdaGrid), i64, vp, vp, i64, i64,
                                            vp, vp, vp, vp, vp, vp]
     L.sdcgym_full_solve_counts.restype = ctypes.c_int
+    L.sdcgym_full_solve_counts_population.argtypes = [ctypes.POINTER(EnvDesc), ctypes.POINTER(LambdaGrid), i64, vp,
+                                                      i64, vp, i64, i64, vp, vp]
+    L.sdcgym_full_solve_counts_population.restype = ctypes.c_int
+    L.sdcgym_spectral_radius_grad_sum_population.argtypes = [dp_, i64, vp, i64, vp, i64, vp, vp, vp]
+    L.sdcgym_spectral_radius_grad_sum_population.restype = ctypes.c_int
     L.sdcgym_vecnorm_scratch_doubles.argtypes = [ctypes.c_int]
     L.sdcgym_vecnorm_accumulate.argtypes = [ctypes.c_int, i64, i64, vp, vp, vp, vp, vp]
     L.sdcgym_vecnorm_merge.argtypes = [ctypes.c_int, dbl, vp, vp, vp, vp, vp]

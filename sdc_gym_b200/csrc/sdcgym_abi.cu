@@ -12,7 +12,10 @@
     extern "C" int sdcgym_launch_step_m##m(const sdcgym_env_desc*, const sdcgym_state*, const sdcgym_step_io*, void*);   \
     extern "C" int sdcgym_launch_full_solve_counts_m##m(const sdcgym_env_desc*, const sdcgym_lambda_grid*, int64_t,      \
                                                         const double*, const double*, int64_t, int64_t, int32_t*,       \
-                                                        double*, uint8_t*, double*, int64_t*, void*);
+                                                        double*, uint8_t*, double*, int64_t*, void*);       \
+    extern "C" int sdcgym_launch_full_solve_counts_population_m##m(const sdcgym_env_desc*, const sdcgym_lambda_grid*, \
+                                                                   int64_t, const double*, int64_t, const double*,    \
+                                                                   int64_t, int64_t, int64_t*, void*);
 SDCGYM_DECL_M(2)
 SDCGYM_DECL_M(3)
 SDCGYM_DECL_M(4)
@@ -216,6 +219,29 @@ extern "C" int sdcgym_full_solve_counts(const sdcgym_env_desc* d, const sdcgym_l
     if (N == 0) return 0;
     switch (d->M) {
 #define C(m) case m: return sdcgym_launch_full_solve_counts_m##m(d, g, N, lam, action, a_es, a_cs, niter_out, residual_out, flags_out, lam_out, hist, stream);
+        C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(9)
+#undef C
+    }
+    return SDCGYM_EUNSUPPORTED;
+}
+
+extern "C" int sdcgym_full_solve_counts_population(const sdcgym_env_desc* d, const sdcgym_lambda_grid* g, int64_t N,
+                                                   const double* lam, int64_t P, const double* action, int64_t a_rs,
+                                                   int64_t a_cs, int64_t* hist, void* stream) {
+    if (!d || !hist || !action) return SDCGYM_ENULL;
+    if (d->env_kind != SDCGYM_ENV_FULL || !sdcgym_supported(d->M, d->prec_type) || d->prec_type == SDCGYM_PREC_FIXED)
+        return SDCGYM_EUNSUPPORTED;
+    if (d->blas_variant != SDCGYM_BLAS_SKYLAKEX && d->blas_variant != SDCGYM_BLAS_HASWELL) return SDCGYM_EUNSUPPORTED;
+    if (P < 1 || N < 0 || d->max_iters < 0 || d->max_iters > kMaxCountIters) return SDCGYM_EINVAL;
+    if (N > 0 && !g && !lam) return SDCGYM_ENULL;
+    if (N > 0 && g && (g->n_re <= 0 || g->n_im <= 0 || g->first < 0 || g->first > g->n_re * g->n_im - N))
+        return SDCGYM_EINVAL;
+    cudaStream_t s = (cudaStream_t)stream;
+    const cudaError_t e = cudaMemsetAsync(hist, 0, (size_t)P * (size_t)(d->max_iters + 3) * sizeof(int64_t), s);
+    if (e != cudaSuccess) return (int)e;
+    if (N == 0) return 0;
+    switch (d->M) {
+#define C(m) case m: return sdcgym_launch_full_solve_counts_population_m##m(d, g, N, lam, P, action, a_rs, a_cs, hist, stream);
         C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(9)
 #undef C
     }

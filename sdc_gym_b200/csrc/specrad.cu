@@ -59,6 +59,48 @@ __global__ void __launch_bounds__(128, (M <= 5) ? 2 : 1) rho_grad_sum_kernel(con
     }
 }
 
+// Population form: row y = blockIdx.y at p.qd + y * qd_rs writes the [nv][T] partials of rho_grad_sum_kernel for that
+// row to segments [y * nv, y * nv + nv) of partials [gridDim.y * nv][T].  The body is rho_grad_sum_kernel's with the row
+// offset; it is spelled out because moving that body into a shared device function changes the code nvcc generates
+// for rho_grad_sum_kernel itself.
+template <int M>
+__global__ void __launch_bounds__(128, (M <= 5) ? 2 : 1) rho_grad_sum_population_kernel(
+    const __grid_constant__ RhoParams<M> p, int64_t qd_rs, double* __restrict__ partials) {
+    __shared__ double part[4][1 + M * (M + 1)];
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    double rho;
+    C2 G[M * M];
+    if (!rho_grad_eval<M, true>(p, i, rho, G, (int64_t)blockIdx.y * qd_rs)) {
+        rho = 0.0;
+#pragma unroll
+        for (int k = 0; k < M * M; k++) G[k] = C2{0.0, 0.0};
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    rho = warp_tree_sum(rho);
+    if (lane == 0) part[warp][0] = rho;
+    int k = 0;
+#pragma unroll
+    for (int r = 0; r < M; r++)
+#pragma unroll
+        for (int c = 0; c < M; c++) {
+            if (is_qd_param(p.prec_type, r, c)) {  // uniform over the block
+                const double gr = warp_tree_sum(G[r * M + c].r), gi = warp_tree_sum(G[r * M + c].i);
+                if (lane == 0) {
+                    part[warp][1 + 2 * k] = gr;
+                    part[warp][2 + 2 * k] = gi;
+                }
+                k++;
+            }
+        }
+    __syncthreads();
+    const int nv = 1 + 2 * p.n_act;
+    if ((int)threadIdx.x < nv) {
+        const int j = threadIdx.x;
+        partials[((int64_t)blockIdx.y * nv + j) * gridDim.x + blockIdx.x] =
+            (part[0][j] + part[1][j]) + (part[2][j] + part[3][j]);
+    }
+}
+
 // in [nv][T] -> out [nv][ceil(T / kFold)]: block (b, j) folds in[j][b*kFold .. b*kFold + kFold) by a balanced tree
 __global__ void __launch_bounds__(kFold) rho_grad_sum_fold_kernel(int64_t T, const double* __restrict__ in,
                                                                    double* __restrict__ out) {
@@ -96,6 +138,27 @@ static int launch_rho_grad_sum(const sdcgym_rho_desc* d, int64_t N, const double
     const int64_t T = (N + 127) / 128;
     rho_grad_sum_kernel<M><<<(unsigned)T, 128, 0, s>>>(p, scratch);
     return grad_sum_fold(T, 1 + 2 * p.n_act, scratch, sums, s);
+}
+
+// P rows in launches of at most 65535 / nv rows (the fold's gridDim.y is rows * nv); each launch folds its rows' P * nv
+// segments like the single-row call folds its nv, in its own share of the scratch (P times the single-row size)
+template <int M>
+static int launch_rho_grad_sum_population(const sdcgym_rho_desc* d, int64_t N, const double* lam, int64_t P,
+                                          const double* qd, int64_t qd_rs, double* scratch, double* sums,
+                                          cudaStream_t s) {
+    RhoParams<M> p;
+    fill_rho_params<M>(p, d, N, lam, qd, nullptr);
+    const int nv = 1 + 2 * p.n_act;
+    const int64_t T = (N + 127) / 128, per_row = nv * grad_sum_scratch_values(N), chunk = 65535 / nv;
+    for (int64_t r0 = 0; r0 < P; r0 += chunk) {
+        const int64_t rows = P - r0 < chunk ? P - r0 : chunk;
+        p.qd = qd + r0 * qd_rs;
+        double* part = scratch + r0 * per_row;
+        rho_grad_sum_population_kernel<M><<<dim3((unsigned)T, (unsigned)rows), 128, 0, s>>>(p, qd_rs, part);
+        const int e = grad_sum_fold(T, (int)(rows * nv), part, sums + r0 * nv, s);
+        if (e) return e;
+    }
+    return 0;
 }
 
 int grad_sum_fold(int64_t T, int nv, double* scratch, double* sums, cudaStream_t s) {
@@ -194,6 +257,27 @@ extern "C" int sdcgym_spectral_radius_grad_sum(const sdcgym_rho_desc* d, int64_t
         return (int)cudaMemsetAsync(sums, 0, (1 + 2 * (size_t)sdcgym_num_actions(d->M, d->prec_type)) * sizeof(double), s);
     switch (d->M) {
 #define C(m) case m: return launch_rho_grad_sum<m>(d, N, lam, qd, rho, scratch, sums, s);
+        C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(9)
+#undef C
+    }
+    return SDCGYM_EUNSUPPORTED;
+}
+
+extern "C" int sdcgym_spectral_radius_grad_sum_population(const sdcgym_rho_desc* d, int64_t N, const double* lam,
+                                                          int64_t P, const double* qd, int64_t qd_rs, double* scratch,
+                                                          double* sums, void* stream) {
+    if (!d || !qd || !scratch || !sums) return SDCGYM_ENULL;
+    if (!sdcgym_supported(d->M, d->prec_type) || d->prec_type == SDCGYM_PREC_FIXED) return SDCGYM_EUNSUPPORTED;
+    if (!d->qd_broadcast || P < 1 || N < 0) return SDCGYM_EINVAL;
+    if (N > 0 && !lam &&
+        (d->grid_re <= 0 || d->grid_im <= 0 || d->grid_first < 0 || d->grid_first + N > d->grid_re * d->grid_im))
+        return SDCGYM_EINVAL;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (N == 0)
+        return (int)cudaMemsetAsync(
+            sums, 0, (size_t)P * (1 + 2 * (size_t)sdcgym_num_actions(d->M, d->prec_type)) * sizeof(double), s);
+    switch (d->M) {
+#define C(m) case m: return launch_rho_grad_sum_population<m>(d, N, lam, P, qd, qd_rs, scratch, sums, s);
         C(2) C(3) C(4) C(5) C(6) C(7) C(8) C(9)
 #undef C
     }

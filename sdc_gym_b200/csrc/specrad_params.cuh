@@ -43,8 +43,10 @@ SDCGYM_HD void grid_lambda(const P& p, int64_t g, double& lr, double& li) {
     li = (p.grid_im > 1) ? p.im_lo + (p.im_hi - p.im_lo) * ((double)b / (double)(p.grid_im - 1)) : p.im_lo;
 }
 
-template <int M>
-SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& li, C2 (&Qd)[M * M]) {
+// ROW: the parameter row is p.qd + qd_off for every sample (a population row, sdcgym_spectral_radius_grad_sum_population)
+template <int M, bool ROW = false>
+SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& li, C2 (&Qd)[M * M],
+                          int64_t qd_off = 0) {
     if (i >= p.N) return false;
     if (p.lam) {
         lr = p.lam[2 * i];
@@ -53,7 +55,7 @@ SDCGYM_HD bool rho_inputs(const RhoParams<M>& p, int64_t i, double& lr, double& 
         grid_lambda(p, p.grid_first + i, lr, li);
     }
     const int w = p.qd_is_complex ? 2 : 1;
-    const double* row = p.qd ? p.qd + (p.qd_broadcast ? 0 : i * (int64_t)p.n_act * w) : nullptr;
+    const double* row = p.qd ? p.qd + (ROW ? qd_off : (p.qd_broadcast ? 0 : i * (int64_t)p.n_act * w)) : nullptr;
     int k = 0;
 #pragma unroll
     for (int r = 0; r < M; r++)
@@ -90,11 +92,11 @@ SDCGYM_HD void rho_one(const RhoParams<M>& p, int64_t i) {
 }
 
 // rho of sample i and G = d rho / d Qd (dense, spectral_radius_grad_one); false past the end of the batch.
-template <int M>
-SDCGYM_HD bool rho_grad_eval(const RhoParams<M>& p, int64_t i, double& rho, C2 (&G)[M * M]) {
+template <int M, bool ROW = false>
+SDCGYM_HD bool rho_grad_eval(const RhoParams<M>& p, int64_t i, double& rho, C2 (&G)[M * M], int64_t qd_off = 0) {
     double lr, li;
     C2 Qd[M * M];
-    if (!rho_inputs<M>(p, i, lr, li, Qd)) return false;
+    if (!rho_inputs<M, ROW>(p, i, lr, li, Qd, qd_off)) return false;
     rho = spectral_radius_grad_one<M>(p.Q, lr * p.dt, li * p.dt, Qd, G);
     return true;
 }

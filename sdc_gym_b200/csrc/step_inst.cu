@@ -3,6 +3,7 @@
 // Exposes sdcgym_launch_reset_m<M> / sdcgym_launch_step_m<M>, dispatched from sdcgym_abi.cu.
 #include <atomic>
 #include <cstdlib>
+#include <type_traits>
 
 #include "step_params.cuh"
 #include "team_kernels.cuh"
@@ -278,14 +279,20 @@ static cudaError_t launch_certified_diag(const StepParams<kM>& p, const FastWork
 }
 
 // sdcgym_full_solve_counts: the per-thread kernel of launch_step at HoldPolicy's residency for every M (the team kernel
-// and the phased solve give the same bits and are not used), plus the histogram behind the side store
-template <int V, bool DENSE>
-static cudaError_t launch_full_solve_counts(const StepParams<kM>& p, const ResetEval& src, int64_t* hist, cudaStream_t s) {
+// and the phased solve give the same bits and are not used), plus the histogram behind the side store.  With
+// PopulationEval, `rows` rows of the population (gridDim.y), hist [rows][max_iters + 3].
+template <int V, bool DENSE, class Src>
+static cudaError_t launch_full_solve_counts(const StepParams<kM>& p, const Src& src, int64_t* hist, cudaStream_t s,
+                                            unsigned rows = 1) {
     constexpr int hold = DENSE ? kHoldDense : kHoldDiag;
     constexpr int minb = DENSE ? HoldPolicy<kM>::dense_minb : HoldPolicy<kM>::diag_minb;
     constexpr int block = DENSE ? HoldPolicy<kM>::dense_block : HoldPolicy<kM>::diag_block;
+    constexpr bool kPop = std::is_same<Src, PopulationEval>::value;
     const size_t smem = step_kernel_smem_bytes<kM, hold, block>() + (hist ? (size_t)(p.max_iters + 3) * sizeof(int) : 0);
-    auto kernel = full_solve_counts_kernel<kM, V, DENSE, hold, minb, block>;
+    auto kernel = [] {
+        if constexpr (kPop) return full_solve_counts_population_kernel<kM, V, DENSE, hold, minb, block>;
+        else return full_solve_counts_kernel<kM, V, DENSE, hold, minb, block>;
+    }();
     if (smem > 48 * 1024) {
         // per-device opt-in, raised when a call needs more than the largest size granted so far
         static std::atomic<size_t> granted[64];
@@ -298,7 +305,8 @@ static cudaError_t launch_full_solve_counts(const StepParams<kM>& p, const Reset
             if (dev >= 0 && dev < 64) granted[dev].store(smem, std::memory_order_relaxed);
         }
     }
-    kernel<<<(unsigned)((p.N + block - 1) / block), block, smem, s>>>(p, src, reinterpret_cast<unsigned long long*>(hist));
+    kernel<<<dim3((unsigned)((p.N + block - 1) / block), rows), block, smem, s>>>(
+        p, src, reinterpret_cast<unsigned long long*>(hist));
     return cudaGetLastError();
 }
 
@@ -306,24 +314,19 @@ static cudaError_t launch_full_solve_counts(const StepParams<kM>& p, const Reset
 
 using namespace sdcgym;
 
-extern "C" int SDCGYM_CAT(sdcgym_launch_full_solve_counts_m, SDCGYM_M)(
-    const sdcgym_env_desc* d, const sdcgym_lambda_grid* g, int64_t N, const double* lam, const double* action,
-    int64_t a_es, int64_t a_cs, int32_t* niter_out, double* residual_out, uint8_t* flags_out, double* lam_out,
-    int64_t* hist, void* stream) {
-    sdcgym_state st{};  // no env state: every plane NULL
+namespace sdcgym {
+
+// StepParams and the lambda source of sdcgym_full_solve_counts(_population): no env state, every plane NULL
+static void fill_counts(StepParams<kM>& p, ResetEval& src, const sdcgym_env_desc* d, const sdcgym_lambda_grid* g,
+                        int64_t N, const double* lam, const double* action, int64_t a_es, int64_t a_cs) {
+    sdcgym_state st{};
     st.N = st.ld = N;
-    StepParams<kM> p;
     fill_params<kM>(p, d, &st);
     p.action = action;
     p.a_es = a_es;
     p.a_cs = a_cs;
-    p.info_niter = niter_out;
-    p.info_res = residual_out;
-    p.flags = flags_out;
-    p.info_lam = lam_out;
     p.autoreset = 0;
     p.strategy = SDCGYM_REW_ITERATION_ONLY;
-    ResetEval src{};
     src.lam = g ? nullptr : lam;
     if (g) {
         src.grid_re = g->n_re;
@@ -334,6 +337,11 @@ extern "C" int SDCGYM_CAT(sdcgym_launch_full_solve_counts_m, SDCGYM_M)(
         src.im_lo = g->im_lo;
         src.im_hi = g->im_hi;
     }
+}
+
+template <class Src>
+static cudaError_t dispatch_full_solve_counts(const sdcgym_env_desc* d, const StepParams<kM>& p, const Src& src,
+                                              int64_t* hist, cudaStream_t s, unsigned rows = 1) {
     bool dense = d->prec_type != SDCGYM_PREC_DIAG;
     if (d->prec_type == SDCGYM_PREC_FIXED) {  // a fixed diagonal matrix takes the diagonal kernel, as in sdcgym_step
         bool diagonal = true;
@@ -342,13 +350,46 @@ extern "C" int SDCGYM_CAT(sdcgym_launch_full_solve_counts_m, SDCGYM_M)(
                 if (r != c && d->Qd_fixed[r * kM + c] != 0.0) diagonal = false;
         dense = !diagonal;
     }
-    cudaStream_t s = (cudaStream_t)stream;
-    cudaError_t e;
     if (d->blas_variant == SDCGYM_BLAS_SKYLAKEX)
-        e = dense ? launch_full_solve_counts<0, true>(p, src, hist, s) : launch_full_solve_counts<0, false>(p, src, hist, s);
-    else
-        e = dense ? launch_full_solve_counts<1, true>(p, src, hist, s) : launch_full_solve_counts<1, false>(p, src, hist, s);
-    return (int)e;
+        return dense ? launch_full_solve_counts<0, true>(p, src, hist, s, rows)
+                     : launch_full_solve_counts<0, false>(p, src, hist, s, rows);
+    return dense ? launch_full_solve_counts<1, true>(p, src, hist, s, rows)
+                 : launch_full_solve_counts<1, false>(p, src, hist, s, rows);
+}
+
+}  // namespace sdcgym
+
+extern "C" int SDCGYM_CAT(sdcgym_launch_full_solve_counts_m, SDCGYM_M)(
+    const sdcgym_env_desc* d, const sdcgym_lambda_grid* g, int64_t N, const double* lam, const double* action,
+    int64_t a_es, int64_t a_cs, int32_t* niter_out, double* residual_out, uint8_t* flags_out, double* lam_out,
+    int64_t* hist, void* stream) {
+    StepParams<kM> p;
+    ResetEval src{};
+    fill_counts(p, src, d, g, N, lam, action, a_es, a_cs);
+    p.info_niter = niter_out;
+    p.info_res = residual_out;
+    p.flags = flags_out;
+    p.info_lam = lam_out;
+    return (int)dispatch_full_solve_counts(d, p, src, hist, (cudaStream_t)stream);
+}
+
+// P rows in launches of at most 65535 (gridDim.y), each row's histogram at hist + row * (max_iters + 3)
+extern "C" int SDCGYM_CAT(sdcgym_launch_full_solve_counts_population_m, SDCGYM_M)(
+    const sdcgym_env_desc* d, const sdcgym_lambda_grid* g, int64_t N, const double* lam, int64_t P,
+    const double* action, int64_t a_rs, int64_t a_cs, int64_t* hist, void* stream) {
+    constexpr int64_t kMaxRows = 65535;
+    StepParams<kM> p;
+    PopulationEval src{};
+    fill_counts(p, src, d, g, N, lam, action, 0, a_cs);
+    src.a_rs = a_rs;
+    for (int64_t r0 = 0; r0 < P; r0 += kMaxRows) {
+        const int64_t rows = P - r0 < kMaxRows ? P - r0 : kMaxRows;
+        p.action = action + r0 * a_rs;
+        const cudaError_t e = dispatch_full_solve_counts(d, p, src, hist + r0 * (int64_t)(d->max_iters + 3),
+                                                         (cudaStream_t)stream, (unsigned)rows);
+        if (e != cudaSuccess) return (int)e;
+    }
+    return 0;
 }
 
 extern "C" int SDCGYM_CAT(sdcgym_launch_reset_m, SDCGYM_M)(const sdcgym_env_desc* d, const sdcgym_state* st,

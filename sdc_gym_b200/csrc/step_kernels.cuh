@@ -374,6 +374,7 @@ struct EnvPlanes {
     static constexpr bool kEval = false;
     SDCGYM_HD void lambda(int64_t, double&, double&) const {}
     SDCGYM_HD void count(bool, int, bool, bool, int) const {}
+    SDCGYM_HD const double* action(const double* a) const { return a; }  // base of the action rows: StepParams::action
 };
 
 // Evaluation of the sdc-v0 full solve from the reset state (sdcgym_full_solve_counts): lambda from an interleaved list
@@ -408,6 +409,16 @@ struct ResetEval {
         hist[bin]++;
 #endif
     }
+    SDCGYM_HD const double* action(const double* a) const { return a; }
+};
+
+// ResetEval for a population of shared action rows (sdcgym_full_solve_counts_population): the block's row is
+// blockIdx.y, at StepParams::action + blockIdx.y * a_rs, and every node reads it as one shared row (a_es = 0).  `row`
+// is set per block by the kernel, so StepParams stays in the constant bank.
+struct PopulationEval : ResetEval {
+    int64_t a_rs;       // doubles between the starts of consecutive rows
+    const double* row;  // this block's row
+    SDCGYM_HD const double* action(const double*) const { return row; }
 };
 
 // `after_loads` runs once every input of the env sits in registers (non-dense kernels): the streaming kernel releases
@@ -459,8 +470,8 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
                     araw[k] = in->action[ii * p.a_es + k * p.a_cs];
                     if (p.is_complex) aimg[k] = in->action[ii * p.a_es + k * p.a_cs + 1];
                 } else {
-                    araw[k] = ld_ro(p.action + i * p.a_es + k * p.a_cs);
-                    if (p.is_complex) aimg[k] = ld_ro(p.action + i * p.a_es + k * p.a_cs + 1);
+                    araw[k] = ld_ro(src.action(p.action) + i * p.a_es + k * p.a_cs);
+                    if (p.is_complex) aimg[k] = ld_ro(src.action(p.action) + i * p.a_es + k * p.a_cs + 1);
                 }
             }
         }
@@ -471,8 +482,8 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
         // env, too many to hold next to the LU factors): without this the first pass over P is a chain of exposed
         // load latencies (ncu: 14 % of the samples of the M = 5 lower_tri kernel on the first load uses).  Pull the
         // row's cache lines into L1 now; the loads below then hit.
-        if (p.action && p.prec_type != SDCGYM_PREC_FIXED) {
-            const double* row = p.action + i * p.a_es;
+        if (src.action(p.action) && p.prec_type != SDCGYM_PREC_FIXED) {
+            const double* row = src.action(p.action) + i * p.a_es;
             constexpr int kMaxLines = (M * (M + 1) * 8 + 127) / 128 + 1;  // complex lower_tri row, unaligned start
             const int64_t row_doubles = p.a_es < (int64_t)M * (M + 1) ? p.a_es : (int64_t)M * (M + 1);
 #pragma unroll
@@ -571,10 +582,10 @@ SDCGYM_HD void step_one(const StepParams<M>& p, const int64_t tid, double* side 
                 d.re = p.Qd[r * M + c];
             } else if (k >= 0) {
                 if (p.is_complex) {
-                    d.re = ld_ro(p.action + i * p.a_es + k * p.a_cs);
-                    d.im = ld_ro(p.action + i * p.a_es + k * p.a_cs + 1);
+                    d.re = ld_ro(src.action(p.action) + i * p.a_es + k * p.a_cs);
+                    d.im = ld_ro(src.action(p.action) + i * p.a_es + k * p.a_cs + 1);
                 } else {
-                    const double a = ld_ro(p.action + i * p.a_es + k * p.a_cs);
+                    const double a = ld_ro(src.action(p.action) + i * p.a_es + k * p.a_cs);
                     d.re = a;
                     if (p.do_scale & SDCGYM_ACTION_SCALE) d.re = (a <= -1.0) ? 0.0 : ((a >= 1.0) ? 1.0 : dmul(0.5, dadd(a, 1.0)));
                 }
@@ -1119,6 +1130,39 @@ __global__ void __launch_bounds__(BLOCK, MINB) full_solve_counts_kernel(const __
         for (int k = threadIdx.x; k < nbins; k += BLOCK)
             if (ev.hist[k]) atomicAdd(hist + k, (unsigned long long)ev.hist[k]);
     }
+}
+
+// sdcgym_full_solve_counts_population: full_solve_counts_kernel for each row of a population, row blockIdx.y at
+// p.action + blockIdx.y * src.a_rs (p.a_es = 0), its histogram (required) at hist + blockIdx.y * (max_iters + 3).
+// Block (x, y) runs what block x of full_solve_counts_kernel runs for that one row.  The body is that kernel's, spelled
+// out: moving it into a shared device function changes the code nvcc generates for full_solve_counts_kernel.
+template <int M, int V, bool DENSE, int HOLD, int MINB, int BLOCK>
+__global__ void __launch_bounds__(BLOCK, MINB) full_solve_counts_population_kernel(
+    const __grid_constant__ StepParams<M> p, const __grid_constant__ PopulationEval src,
+    unsigned long long* __restrict__ hist) {
+    extern __shared__ double2 eval_smem[];  // [side store of HOLD][BLOCK], then the block's histogram (int)
+    constexpr size_t kSide = step_kernel_smem_bytes<M, HOLD, BLOCK>() / sizeof(double2);
+    const int nbins = p.max_iters + 3;
+    PopulationEval ev = src;
+    ev.row = p.action + (int64_t)blockIdx.y * src.a_rs;
+    ev.hist = reinterpret_cast<int*>(eval_smem + kSide);
+    hist += (int64_t)blockIdx.y * nbins;
+    for (int k = threadIdx.x; k < nbins; k += BLOCK) ev.hist[k] = 0;
+    __syncthreads();
+    const int64_t tid = (int64_t)blockIdx.x * BLOCK + threadIdx.x;
+    if constexpr (HOLD == 5 || HOLD == 7) {
+        step_one<M, SDCGYM_ENV_FULL, V, DENSE, HOLD, NoAfterLoads, 0, PopulationEval>(
+            p, tid, nullptr, 1, reinterpret_cast<cplx*>(eval_smem) + threadIdx.x, BLOCK, nullptr, NoAfterLoads(), 0, ev);
+    } else if constexpr (HOLD >= 3) {
+        step_one<M, SDCGYM_ENV_FULL, V, DENSE, HOLD, NoAfterLoads, 0, PopulationEval>(
+            p, tid, reinterpret_cast<double*>(eval_smem) + threadIdx.x, BLOCK, nullptr, 1, nullptr, NoAfterLoads(), 0, ev);
+    } else {
+        step_one<M, SDCGYM_ENV_FULL, V, DENSE, HOLD, NoAfterLoads, 0, PopulationEval>(
+            p, tid, nullptr, 1, nullptr, 1, nullptr, NoAfterLoads(), 0, ev);
+    }
+    __syncthreads();  // (every thread comes back from step_one: its exits are returns of the inlined body)
+    for (int k = threadIdx.x; k < nbins; k += BLOCK)
+        if (ev.hist[k]) atomicAdd(hist + k, (unsigned long long)ev.hist[k]);
 }
 #endif
 

@@ -26,6 +26,19 @@ def _torch():
     return torch
 
 
+def count_stats(hist, max_iters):
+    """``test_model``'s numbers from histograms ``hist`` (numpy int64 [..., max_iters + 3]), each a numpy array over
+    the leading axes: (count, n_err, n_exhausted, n_success, success_rate, mean_niter).  Success is a converged episode
+    whose niter is below 50; ``mean_niter`` is 666.0 where nothing succeeds and ``success_rate`` 0.0 for an empty set."""
+    h = np.asarray(hist)
+    ns = min(MAX_ITERS, max_iters + 1)
+    count = h.sum(-1)
+    n_success = h[..., :ns].sum(-1)
+    rate = np.where(count > 0, n_success / np.maximum(count, 1), 0.0)
+    mean = np.where(n_success > 0, np.sum(np.arange(ns) * h[..., :ns], -1) / np.maximum(n_success, 1), 666.0)
+    return count, h[..., max_iters + 1], h[..., max_iters + 2], n_success, rate, mean
+
+
 class CountSummary:
     """What ``test_model`` reports for a set of episodes, from the device histogram ``hist_device`` (int64
     [max_iters + 3]: niter of the converged episodes, then the err count, then the count of episodes that ran out of
@@ -48,37 +61,73 @@ class CountSummary:
             self._hist = self.hist_device.cpu().numpy()
         return self._hist
 
+    def _stats(self):
+        return count_stats(self.hist, self.max_iters)
+
     @property
     def n_err(self):
-        return int(self.hist[self.max_iters + 1])
+        return int(self._stats()[1])
 
     @property
     def n_exhausted(self):
-        return int(self.hist[self.max_iters + 2])
+        return int(self._stats()[2])
 
     @property
     def count(self):
-        return int(self.hist.sum())
+        return int(self._stats()[0])
 
     @property
     def n_success(self):
-        return int(self.hist[:min(MAX_ITERS, self.max_iters + 1)].sum())
+        return int(self._stats()[3])
 
     @property
     def success_rate(self):
-        return self.n_success / self.count if self.count else 0.0
+        return float(self._stats()[4])
 
     @property
     def mean_niter(self):
-        n = self.n_success
-        if n == 0:
-            return 666
-        k = np.arange(min(MAX_ITERS, self.max_iters + 1))
-        return int(np.sum(k * self.hist[: len(k)])) / n
+        mean = float(self._stats()[5])
+        return 666 if self.n_success == 0 else mean
 
     def __repr__(self):
         return (f"CountSummary(count={self.count}, success_rate={self.success_rate:.6f}, "
                 f"mean_niter={self.mean_niter}, n_err={self.n_err}, n_exhausted={self.n_exhausted})")
+
+
+class PopulationSummary:
+    """``CountSummary`` for each of P action rows, from the device histograms ``hist_device`` (int64
+    [P, max_iters + 3]), copied to the host once, on first use.  ``count``, ``n_err``, ``n_exhausted``,
+    ``n_success``, ``success_rate`` and ``mean_niter`` are numpy arrays (P,) with ``CountSummary``'s rules (666.0
+    where nothing succeeds); ``summary[p]`` is row p's ``CountSummary``."""
+
+    def __init__(self, hist_device, max_iters=MAX_ITERS):
+        self.hist_device = hist_device
+        self.max_iters = int(max_iters)
+        self._hist = None
+
+    def __len__(self):
+        return int(self.hist_device.shape[0])
+
+    @property
+    def hist(self):
+        if self._hist is None:
+            self._hist = self.hist_device.cpu().numpy()
+        return self._hist
+
+    def __getitem__(self, p):
+        s = CountSummary(self.hist_device[p], self.max_iters)
+        s._hist = self.hist[p]
+        return s
+
+    count = property(lambda self: count_stats(self.hist, self.max_iters)[0])
+    n_err = property(lambda self: count_stats(self.hist, self.max_iters)[1])
+    n_exhausted = property(lambda self: count_stats(self.hist, self.max_iters)[2])
+    n_success = property(lambda self: count_stats(self.hist, self.max_iters)[3])
+    success_rate = property(lambda self: count_stats(self.hist, self.max_iters)[4])
+    mean_niter = property(lambda self: count_stats(self.hist, self.max_iters)[5])
+
+    def __repr__(self):
+        return f"PopulationSummary(P={len(self)}, success_rate={self.success_rate}, mean_niter={self.mean_niter})"
 
 
 class IterationCounts:
@@ -130,20 +179,31 @@ class IterationCounts:
     def _stream(self):
         return ctypes.c_void_p(_torch().cuda.current_stream(self.device).cuda_stream)
 
+    def _action_tensor(self, actions):
+        torch = _torch()
+        t = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.array(actions))
+        if not (t.is_floating_point() or t.is_complex()):
+            raise TypeError(f"actions must be real or complex floating point, not {t.dtype}")
+        if t.is_complex() and not self.free_action_space:
+            raise TypeError("complex actions need free_action_space=True")
+        return t
+
+    def _device_rows(self, t):
+        """the rows as step_tensor reads them: complex128 (viewed as pairs) with free_action_space, else float64"""
+        torch = _torch()
+        t = t.to(self.device)
+        return torch.view_as_real(t.to(torch.complex128).contiguous()) if self.free_action_space \
+            else t.to(torch.float64).contiguous()
+
     def _rows(self, actions, N, grid):
         """(tensor kept alive, pointer, env stride, component stride) of the action rows, as step_tensor reads them"""
-        torch = _torch()
         if self.prec is not None:
             if actions is not None:
                 raise ValueError(f"prec={self.prec!r} fixes Q_delta: no actions")
             return None, None, 0, 0
         if actions is None:
             raise ValueError("actions required (no fixed prec)")
-        t = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.array(actions))
-        if not (t.is_floating_point() or t.is_complex()):
-            raise TypeError(f"actions must be real or complex floating point, not {t.dtype}")
-        if t.is_complex() and not self.free_action_space:
-            raise TypeError("complex actions need free_action_space=True")
+        t = self._action_tensor(actions)
         if t.dim() == 1:
             t = t.reshape(1, -1)
         if t.dim() != 2 or t.shape[1] != self.n_act:
@@ -152,10 +212,31 @@ class IterationCounts:
         if not shared and (grid or t.shape[0] != N):
             raise ValueError(f"actions must be one row ({self.n_act},) in grid mode" if grid else
                              f"actions must have shape ({N}, {self.n_act}) or ({self.n_act},)")
-        t = t.to(self.device)
-        a = torch.view_as_real(t.to(torch.complex128).contiguous()) if self.free_action_space \
-            else t.to(torch.float64).contiguous()
+        a = self._device_rows(t)
         return a, a.data_ptr(), 0 if shared else a.stride(0), a.stride(1)
+
+    def _population(self, population):
+        """(tensor kept alive, row stride, component stride) of P candidate rows (P, n_act)"""
+        if self.prec is not None:
+            raise ValueError(f"prec={self.prec!r} fixes Q_delta: a population has no rows")
+        t = self._action_tensor(population)
+        if t.dim() != 2 or t.shape[0] < 1 or t.shape[1] != self.n_act:
+            raise ValueError(f"population must have shape (P, {self.n_act}) with P >= 1, not {tuple(t.shape)}")
+        a = self._device_rows(t)
+        return a, a.stride(0), a.stride(1)
+
+    def _run_population(self, N, lam_r, grid, population):
+        """hist (P, max_iters + 3) of sdcgym_full_solve_counts_population"""
+        torch = _torch()
+        a, rs, cs = self._population(population)
+        P = a.shape[0]
+        hist = torch.empty((P, self.max_iters + 3), dtype=torch.int64, device=self.device)
+        _lib.check(self._L.sdcgym_full_solve_counts_population(
+            ctypes.byref(self._desc), None if grid is None else ctypes.byref(grid), N,
+            None if lam_r is None else lam_r.data_ptr(), P, a.data_ptr(), rs, cs, hist.data_ptr(), self._stream()),
+            "sdcgym_full_solve_counts_population")
+        self._keep = (a, lam_r)
+        return hist
 
     def _lams(self, lams):
         torch = _torch()
@@ -245,3 +326,25 @@ class IterationCounts:
 
         hist, _ = _dist.sharded_rows_sum(n_re, rows, lambda lo, hi: rows_hist(self, lo, hi))
         return CountSummary(hist, self.max_iters)
+
+    @_lib.on_device
+    def population_summary(self, lams, population):
+        """``summary`` for each row of ``population`` (P, n_act), every row shared by all lambdas, in one launch
+        (``sdcgym_full_solve_counts_population``).  Returns a ``PopulationSummary``; row p equals ``summary(lams,
+        population[p])``, bit for bit.  The dtype rules are those of ``summary``."""
+        lam_r = self._lams(lams)
+        return PopulationSummary(self._run_population(lam_r.shape[0], lam_r, None, population), self.max_iters)
+
+    def population_grid_summary(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, population, rows=None):
+        """``grid_summary`` for each row of ``population`` (P, n_act) in one launch per shard.  ``rows=None``: grid rows
+        sharded over the ranks of the default process group with one all-reduce of the (P, max_iters + 3) histograms;
+        ``rows=(lo, hi)``: grid rows lo..hi-1 only, no collective call.  Returns a ``PopulationSummary``."""
+        from . import dist as _dist
+
+        @_lib.on_device
+        def rows_hist(self, lo, hi):
+            g = self._grid(n_re, n_im, lambda_real_interval, lambda_imag_interval, lo)
+            return self._run_population((hi - lo) * int(n_im), None, g, population)  # N = 0 zeroes hist
+
+        hist, _ = _dist.sharded_rows_sum(n_re, rows, lambda lo, hi: rows_hist(self, lo, hi))
+        return PopulationSummary(hist, self.max_iters)

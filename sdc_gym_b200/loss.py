@@ -175,17 +175,18 @@ class SpectralRadiusLoss:
         return sums
 
     def _mean_and_grad(self, sums, count, is_c, convention):
-        """(sums[0] / count, g / count) with g in ``convention`` (see ``value_and_grad``); real rows give a real g."""
+        """(sums[..., 0] / count, g / count) with g in ``convention`` (see ``value_and_grad``); real rows give a real g."""
         torch = _torch()
         if convention not in ("jax", "torch"):
             raise ValueError("convention must be 'jax' or 'torch'")
-        pairs = sums[1:].reshape(self.n_out, 2) / max(count, 1)  # no samples: zero gradient, NaN mean
+        # sums (..., 1 + 2 n_out): one row or a population of rows
+        pairs = sums[..., 1:].reshape(*sums.shape[:-1], self.n_out, 2) / max(count, 1)  # no samples: zero gradient, NaN mean
         g = torch.view_as_complex(pairs.contiguous())
         if not is_c:
             g = g.real.contiguous()
         elif convention == "torch":
             g = g.conj().resolve_conj()
-        return sums[0] / count, g
+        return sums[..., 0] / count, g
 
     def _shared_row(self, output):
         if self.prec is not None:
@@ -216,12 +217,14 @@ class SpectralRadiusLoss:
         return self._mean_and_grad(sums, B, is_c, convention)
 
     @_lib.on_device
-    def _grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of):
-        """sums_of(N) over grid rows lo..hi-1 with the grid set in the descriptor (zeros for an empty range)"""
+    def _grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of, P=None):
+        """sums_of(N) over grid rows lo..hi-1 with the grid set in the descriptor (zeros for an empty range, of shape
+        (P, 1 + 2 n_out) for a population of P rows)"""
         torch = _torch()
         N = (hi - lo) * int(n_im)
         if N == 0:  # an empty shard contributes nothing and launches nothing
-            return torch.zeros(1 + 2 * self.n_out, dtype=torch.float64, device=self.device)
+            shape = (1 + 2 * self.n_out,) if P is None else (P, 1 + 2 * self.n_out)
+            return torch.zeros(shape, dtype=torch.float64, device=self.device)
         d = self._desc
         d.grid_re, d.grid_im, d.grid_first = int(n_re), int(n_im), lo * int(n_im)
         d.re_lo, d.re_hi = float(lambda_real_interval[0]), float(lambda_real_interval[1])
@@ -231,14 +234,15 @@ class SpectralRadiusLoss:
         finally:
             d.grid_first = 0
 
-    def _sharded_grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, rows, sums_of):
+    def _sharded_grid_sums(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, rows, sums_of, P=None):
         """(sums, sample count) of sums_of over the grid: ``rows=None`` shards the rows over the ranks of the default
-        process group and all-reduces the 1 + 2 n_out sums; ``rows=(lo, hi)`` takes those rows only, no collective."""
+        process group and all-reduces the 1 + 2 n_out sums (of each of P rows); ``rows=(lo, hi)`` takes those rows
+        only, no collective."""
         from . import dist as _dist
 
         n_re, n_im = int(n_re), int(n_im)
         sums, n_rows = _dist.sharded_rows_sum(n_re, rows, lambda lo, hi: self._grid_sums(
-            n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of))
+            n_re, n_im, lambda_real_interval, lambda_imag_interval, lo, hi, sums_of, P))
         return sums, n_rows * n_im
 
     def grid_value_and_grad(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, output, rows=None,
@@ -257,6 +261,75 @@ class SpectralRadiusLoss:
         """``grid_value_and_grad`` over the whole grid as a torch scalar that supports ``.backward()`` into the
         parameter row ``output``."""
         return _SharedRowFn.apply(output, lambda o, conv: self.grid_value_and_grad(
+            n_re, n_im, lambda_real_interval, lambda_imag_interval, o, convention=conv))
+
+    # ---- populations: P parameter rows, each shared by every lambda, in one launch ----
+    def _population_rows(self, population):
+        """(qd (P, n_out[, 2]) float64 on the device, is_c) of P >= 1 parameter rows"""
+        torch = _torch()
+        if self.prec is not None:
+            raise ValueError("a fixed preconditioner has no parameters to differentiate")
+        t = population.detach() if isinstance(population, torch.Tensor) else torch.as_tensor(np.array(population))
+        if t.dim() != 2 or t.shape[0] < 1 or t.shape[1] != self.n_out:
+            raise ValueError(f"population must have shape (P, {self.n_out}) with P >= 1, not {tuple(t.shape)}")
+        qd, is_c, _ = self._outputs_tensor(t, t.shape[0])
+        return qd, is_c
+
+    def _population_sums(self, N, lam_r, qd, is_c):
+        """(P, 1 + 2 n_out) CUDA float64 (``sdcgym_spectral_radius_grad_sum_population``): ``_grad_sums`` of each row"""
+        torch = _torch()
+        d = self._desc
+        d.qd_is_complex, d.qd_broadcast = is_c, 1
+        P = qd.shape[0]
+        sums = torch.empty((P, 1 + 2 * self.n_out), dtype=torch.float64, device=self.device)
+        n_scratch = int(self._L.sdcgym_spectral_radius_grad_sum_scratch_doubles(self.M, d.prec_type, N))
+        if n_scratch < 0:
+            _lib.check(n_scratch, "sdcgym_spectral_radius_grad_sum_scratch_doubles")
+        scratch = torch.empty(P * n_scratch, dtype=torch.float64, device=self.device)
+        _lib.check(self._L.sdcgym_spectral_radius_grad_sum_population(
+            ctypes.byref(d), N, None if lam_r is None else lam_r.data_ptr(), P, qd.data_ptr(), qd[0].numel(),
+            scratch.data_ptr(), sums.data_ptr(), self._stream()), "sdcgym_spectral_radius_grad_sum_population")
+        self._keep = (lam_r, qd, scratch)
+        return sums
+
+    @_lib.on_device
+    def population_value_and_grad(self, lams, population, convention="jax"):
+        """``shared_value_and_grad`` for each row of ``population`` (P, n_out), every row shared by all lambdas, in one
+        launch: (means (P,), gradients (P, n_out)); row p equals ``shared_value_and_grad(lams, population[p])`` bit for
+        bit.  An empty batch gives (NaN, zeros) per row."""
+        torch = _torch()
+        qd, is_c = self._population_rows(population)
+        lam = lams if isinstance(lams, torch.Tensor) else torch.as_tensor(np.asarray(lams, dtype=np.complex128))
+        lam = lam.detach().to(self.device).to(torch.complex128).reshape(-1).contiguous()
+        B = lam.numel()
+        if B == 0:  # 0/0, and nothing to launch (a NULL lambda pointer would select grid mode in the ABI)
+            sums = torch.zeros((qd.shape[0], 1 + 2 * self.n_out), dtype=torch.float64, device=self.device)
+        else:
+            d = self._desc
+            d.grid_re = d.grid_im = 0
+            sums = self._population_sums(B, torch.view_as_real(lam), qd, is_c)
+        return self._mean_and_grad(sums, B, is_c, convention)
+
+    def population_grid_value_and_grad(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, population,
+                                       rows=None, convention="jax"):
+        """``grid_value_and_grad`` for each row of ``population`` (P, n_out) in one launch per shard: (means (P,),
+        gradients (P, n_out)).  ``rows=None``: the whole grid, rows sharded over the ranks of the default process
+        group with one all-reduce of P (1 + 2 n_out) doubles; ``rows=(lo, hi)``: grid rows lo..hi-1 only, no
+        collective call (an empty range gives (NaN, zeros) per row)."""
+        qd, is_c = self._population_rows(population)
+        sums, count = self._sharded_grid_sums(n_re, n_im, lambda_real_interval, lambda_imag_interval, rows,
+                                              lambda N: self._population_sums(N, None, qd, is_c), qd.shape[0])
+        return self._mean_and_grad(sums, count, is_c, convention)
+
+    def population_differentiable(self, lams, population):
+        """``population_value_and_grad`` as a (P,) tensor whose ``.sum().backward()`` gives each row of ``population``
+        its own gradient (real rows real, complex rows in the torch convention, as ``differentiable``)"""
+        return _SharedRowFn.apply(population, lambda o, conv: self.population_value_and_grad(lams, o, conv))
+
+    def population_grid_differentiable(self, n_re, n_im, lambda_real_interval, lambda_imag_interval, population):
+        """``population_grid_value_and_grad`` over the whole grid as a (P,) tensor that supports ``.backward()`` into
+        ``population``"""
+        return _SharedRowFn.apply(population, lambda o, conv: self.population_grid_value_and_grad(
             n_re, n_im, lambda_real_interval, lambda_imag_interval, o, convention=conv))
 
     @_lib.on_device
@@ -333,18 +406,21 @@ def _make_shared_row_fn():
     torch = _torch()
 
     class SharedRowFn(torch.autograd.Function):
-        """value_and_grad(row, convention) -> (scalar, g of the row's size): the loss of one shared parameter row"""
+        """value_and_grad(row, convention) -> (scalar, g of the row's size): the loss of one shared parameter row; or
+        (values (P,), g (P, n_out)): the losses of a population of P rows"""
 
         @staticmethod
         def forward(ctx, row, value_and_grad):
             value, g = value_and_grad(row, "torch")
             ctx.save_for_backward(g)
             ctx.out_shape, ctx.out_dtype = row.shape, row.dtype
-            return value.reshape(())
+            return value.reshape(value.shape[:1] if value.dim() else ())
 
         @staticmethod
         def backward(ctx, upstream):
             (g,) = ctx.saved_tensors
+            if upstream.dim():  # one upstream value per population row
+                upstream = upstream[:, None]
             return (g * upstream).reshape(ctx.out_shape).to(ctx.out_dtype), None
 
     return SharedRowFn

@@ -3,7 +3,7 @@
     python tools/sass_identity.py OLD_DIR NEW_DIR [name.o ...]
 
 Each object is disassembled with ``cuobjdump -sass`` and split into functions.  A function of OLD_DIR must have
-identical instructions in NEW_DIR (addresses and encodings included); functions only NEW_DIR has are listed as added.
+identical instructions in NEW_DIR (addresses and encodings included, runs of blanks compared as one); functions only NEW_DIR has are listed as added.
 Exits 1 when a function of OLD_DIR changed or disappeared.
 """
 from __future__ import annotations
@@ -23,7 +23,7 @@ def functions(obj):
             name = m.group(1)
             out[name] = []
         elif name is not None and line.strip():
-            out[name].append(line.strip())
+            out[name].append(" ".join(line.split()))  # (cuobjdump pads columns to the file's longest name)
     return out
 
 
